@@ -2,6 +2,7 @@
 """bench.py -- block-Lanczos mod-p hot path on B200: Lanczos iterations/s and SpMV G(nnz*n)/s.
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload cfg4|cfg4_small|cfg4_tiny]
+                    [--dump-outputs DIR]
 
 A "step" is one block-Lanczos iteration (two n-wide sparse products, block dot products,
 semi-inverse, orthogonalize) of the named workload.  Default workload (BASELINE.json configs[3],
@@ -30,6 +31,9 @@ One JSON line on stdout (rank 0).  Its parts:
   cpu_baseline          the UNMODIFIED reference's builds (oracle/_ref, compiled from /root/reference) on
                         the host cores on a scaled-down twin: OpenMP (timing build), OpenMP at a prime where
                         its deferred modulo is exact, sequential, and its SpMV alone.
+
+--dump-outputs DIR also writes the state after the last timed step as DIR/<name>.npy (see dump_outputs).  The
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -61,6 +65,7 @@ UNIT = "iterations/s"
 CPU_TWIN = dict(rows=200_000, cols=200_000)          # bounded CPU sample of the same generator
 SWEEP_NS = (1, 2, 4, 8, 16, 32)
 SWEEP_PRIMES = (65537, P_MERSENNE)
+DUMP_ROWS = 1 << 16          # rows per block kept by --dump-outputs: 4 blocks x 65536 x n=16 x 8 B = 32 MB
 
 
 def peaks():
@@ -274,7 +279,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip spmv_sweep, small_configs and the tiny-twin parity check")
     ap.add_argument("--sweep-budget-s", type=float, default=100.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the state after the last timed step to DIR/<name>.npy (float64, sampled rows)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        # the reference arm times the CPU program on a scaled-down twin: it has no state of the workload to write
+        ap.error("--dump-outputs is not available with --impl reference")
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
     w = WORKLOADS[a.workload]
     rank = int(os.environ.get("RANK", "0"))
@@ -398,6 +408,8 @@ def main():
     # (blk_get_state is collective: every rank asks for v; rank 0 hashes it)
     ctx.L.blk_get_state(ctx.h, out_np.ctypes.data, None, None, None)
     state_sha256 = hashlib.sha256(out_np[:N * n].tobytes()).hexdigest() if rank == 0 else None
+    if a.dump_outputs:
+        dump_outputs(np, ctx, out_np, n, rank, a.dump_outputs)
 
     # -------- end to end through the C ABI with host buffers
     e2e = None
@@ -521,6 +533,29 @@ def main():
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+def dump_outputs(np, ctx, buf, n, rank, out_dir):
+    """--dump-outputs: what a caller of the timed path receives after its last step, as DIR/<name>.npy in float64
+    (exact for residues < 2^32).  v, tmp, Av, p: the blocks of blk_get_state, as rows x n -- every padded row, or
+    DUMP_ROWS rows drawn with a fixed seed (sorted) when there are more.  vtAv, vtAAv, winv, d: the n x n matrices
+    of that step (blk_get_small).  blk_get_state is collective, so every rank takes part; rank 0 writes.  `buf` is
+    a host buffer of ctx.pad residues."""
+    R = ctx.pad // n
+    rows = np.arange(R) if R <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(R, DUMP_ROWS, replace=False))
+    out = {}
+    for k, name in enumerate(("v", "tmp", "Av", "p")):
+        ptrs = [None] * 4
+        ptrs[k] = buf.ctypes.data
+        ctx._ck(ctx.L.blk_get_state(ctx.h, *ptrs))
+        out[name] = buf.reshape(R, n)[rows]
+    small = ctx.get_small()
+    out.update(vtAv=small["vtAv"].reshape(n, n), vtAAv=small["vtAAv"].reshape(n, n), winv=small["winv"].reshape(n, n),
+               d=small["d"])
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for name, arr in out.items():
+            np.save(os.path.join(out_dir, name + ".npy"), arr.astype(np.float64))
 
 
 def spmv_sweep(B, torch, w, coo, nnz, local_rank, rank, world, new_id, max_over_ranks, stream, peak, budget_s):

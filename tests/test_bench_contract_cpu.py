@@ -35,6 +35,13 @@ def test_non_zero_ranks_of_the_reference_arm_do_nothing():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_reference_arm_rejects_dump_outputs(tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",
+                        "--dump-outputs", str(tmp_path / "d")], capture_output=True, text=True, timeout=60)
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr and r.stdout == ""
+    assert not (tmp_path / "d").exists()
+
+
 def test_dense_roofline_helper():
     import importlib.util
     spec = importlib.util.spec_from_file_location("_bench", os.path.join(ROOT, "bench.py"))
