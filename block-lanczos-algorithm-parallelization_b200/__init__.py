@@ -29,7 +29,7 @@ PHASES = ("spmv1", "spmv2", "dots", "small", "ortho", "exchange")
 ABI_SYMBOLS = (
     "blk_abi_version", "blk_last_error", "blk_device_count", "blk_nccl_unique_id", "blk_create",
     "blk_destroy", "blk_plan_shards", "blk_plan_grid", "blk_block_pad", "blk_set_state", "blk_iterate", "blk_get_state", "blk_get_state_local", "blk_final_check",
-    "blk_check_kernel_block", "blk_get_small",
+    "blk_check_kernel_block", "blk_kernel_basis", "blk_get_small",
     "blk_spmv", "blk_block_dot_products", "blk_semi_inverse", "blk_orthogonalize",
     "blk_set_profiling", "blk_get_phase_times", "blk_time_spmv", "blk_kernel_launches", "blk_get_info",
 )
@@ -89,6 +89,7 @@ def load_library(path: str | None = None) -> C.CDLL:
     L.blk_get_state_local.argtypes = [vp, vp, vp, vp]
     L.blk_final_check.argtypes = [vp, C.POINTER(i32), C.POINTER(i32)]
     L.blk_check_kernel_block.argtypes = [vp, vp, C.POINTER(i32)]
+    L.blk_kernel_basis.argtypes = [vp, vp, C.POINTER(i32)]
     L.blk_get_small.argtypes = [vp, vp, vp, vp, vp, C.POINTER(i32)]
     L.blk_spmv.argtypes = [vp, vp, vp, i32]
     L.blk_block_dot_products.argtypes = [vp, vp, vp, i64, vp, vp]
@@ -305,6 +306,14 @@ class BlockLanczos:
         ok = C.c_int32(0)
         self._ck(self.L.blk_check_kernel_block(self.h, _ptr(x), C.byref(ok)))
         return bool(ok.value)
+
+    def kernel_basis(self) -> np.ndarray:
+        """The kernel vectors inside span(v) (blk_kernel_basis): an N x k uint32 array of independent columns,
+        each annihilated by M (x^T M == 0 for --left, M x == 0 for --right); k may be 0."""
+        x = np.empty(self.N * self.n, dtype=np.uint32)
+        k = C.c_int32(0)
+        self._ck(self.L.blk_kernel_basis(self.h, _ptr(x), C.byref(k)))
+        return x.reshape(self.N, self.n)[:, :k.value].copy()
 
     def get_small(self):
         n = self.n

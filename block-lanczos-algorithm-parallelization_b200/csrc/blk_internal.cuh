@@ -275,3 +275,28 @@ void dense_prepare(const Geometry &geo, const ModP &m);
 // unpad gathers dst row r from src row map[r0 + r]; without a map row r <-> row r of the given pointers.
 int launch_pad_rows(const u32 *src, u32 *dst, int64_t rows, int n, int np, const u32 *map, int64_t r0, cudaStream_t st);
 int launch_unpad_rows(const u32 *src, u32 *dst, int64_t rows, int n, int np, const u32 *map, int64_t r0, cudaStream_t st);
+// kernel_basis.cu: the kernel vectors inside span(v) (blk_kernel_basis).  A record is (n + 1) x n_pad words: word 0 the
+// rank r, rows 1 .. r an echelon basis of a block's row space.
+struct KbArgs {
+        int n = 0, world = 1, ctas = 1;
+        ModP m;
+        const u32 *v = nullptr;        // this rank's rows of v (vrows x n_pad)
+        int64_t vrows = 0;
+        const u32 *t = nullptr;        // this rank's rows of T = S1 v (trows x n_pad)
+        int64_t trows = 0;
+        u32 *part = nullptr;           // [2][ctas][n][n_pad] per-CTA bases
+        int *prank = nullptr;          // [2][ctas]
+        unsigned *counter = nullptr;   // last-CTA ticket (zero before the launch, re-armed by it)
+        u32 *rec_own = nullptr;        // this rank's two records (v, T)
+        u32 *rec_all = nullptr;        // [world][2] records
+        u32 *A = nullptr;              // n_pad x n_pad: A_S, column s = a_f of the s-th vector
+        int *k = nullptr;              // number of kernel vectors
+        u32 *x = nullptr;              // vrows x n_pad: X = v A_S
+};
+int kb_ctas(int64_t rows);
+// k_kb_reduce: both blocks -> rec_own
+int launch_kb_reduce(int np, const KbArgs &a, cudaStream_t st);
+// k_kb_small: rec_all -> A, k
+int launch_kb_small(int np, const KbArgs &a, cudaStream_t st);
+// k_kb_apply: x = v A
+int launch_kb_apply(int np, const KbArgs &a, cudaStream_t st);

@@ -2536,6 +2536,85 @@ int blk_check_kernel_block(blk_ctx *c, const uint32_t *x, int32_t *ok)
         return 0;
 }
 
+// One rank of blk_kernel_basis: its rows of v and T reduced to two records, the records of all ranks gathered
+// (one NCCL all-gather), the n x n stage redundantly on every rank, and X = v A_S for the rows this rank owns.
+// whole: write every row of x (a rank of a multi-process job), else only this rank's rows (group members).
+static int kernel_basis_rank(blk_ctx *c, uint32_t *x, int32_t *k, bool whole)
+{
+        CU(cudaSetDevice(c->device));
+        const int n = c->geo.n, np = c->geo.np;
+        if (c->grid_on && grid_export(c)) return 1;
+        const int64_t n0 = c->n0(), ln = c->n1() - n0, lm = c->m1() - c->m0();
+        // T = S1 v of the current v, exactly as blk_final_check obtains it (v, tmp, Av and p are left as they are)
+        bool have = c->tmp_is_spmv || (c->mg_recur && c->ran_since_set);
+        const size_t rec_words = (size_t)(n + 1) * np;
+        KbArgs a;
+        a.n = n; a.world = c->world; a.m = c->m;
+        a.v = c->v + (size_t)n0 * np; a.vrows = ln;
+        a.t = c->tmp + (size_t)c->m0() * np; a.trows = lm;
+        a.ctas = kb_ctas(std::max(ln, lm));
+        struct Bufs {
+                std::vector<void *> p;
+                ~Bufs() { for (void *q : p) cudaFree(q); }
+        } bufs;
+        auto grab = [&](void **dst, size_t bytes) {
+                cudaError_t e = cudaMalloc(dst, bytes ? bytes : 4);
+                if (e == cudaSuccess) bufs.p.push_back(*dst);
+                return e;
+        };
+        u32 *scratch = nullptr, *xf = nullptr;
+        if (!have) {
+                if (c->world > 1 && allgather_rows(c, c->v, c->n_off)) return 1;
+                CU(grab((void **)&scratch, sizeof(u32) * (size_t)lm * np));
+                c->launches += launch_spmv(c->S1, c->geo, c->m, c->v, scratch, nullptr, c->stream);
+                a.t = scratch;
+        }
+        CU(grab((void **)&a.part, sizeof(u32) * (size_t)2 * a.ctas * n * np));
+        CU(grab((void **)&a.prank, sizeof(int) * (size_t)2 * a.ctas));
+        CU(grab((void **)&a.counter, sizeof(unsigned)));
+        CU(grab((void **)&a.rec_all, sizeof(u32) * (size_t)c->world * 2 * rec_words));
+        CU(grab((void **)&a.A, sizeof(u32) * (size_t)np * np));
+        CU(grab((void **)&a.k, sizeof(int)));
+        CU(grab((void **)&xf, sizeof(u32) * (size_t)gather_cap(c->n_off) * np));
+        a.rec_own = a.rec_all + (size_t)c->rank * 2 * rec_words;
+        a.x = xf + (size_t)n0 * np;
+        CU(cudaMemsetAsync(a.counter, 0, sizeof(unsigned), c->stream));
+        c->launches += launch_kb_reduce(np, a, c->stream);
+        if (c->world > 1)
+                NC(g_nccl.AllGather(a.rec_own, a.rec_all, 2 * rec_words, ncclUint32, c->comm, c->stream));
+        c->launches += launch_kb_small(np, a, c->stream);
+        c->launches += launch_kb_apply(np, a, c->stream);
+        int hk = 0;
+        CU(cudaMemcpyAsync(&hk, a.k, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        CU(cudaGetLastError());
+        // down to the host like v in download_state
+        const bool all = whole && c->world > 1;
+        if (c->relabel_mg()) {
+                const int64_t r0 = all ? 0 : c->h0(), cnt = all ? c->N : c->h1() - c->h0();
+                if (allgather_rows(c, xf, c->n_off)) return 1;
+                if (download_rows(c, x + (size_t)r0 * n, xf, cnt, c->n_old2new, r0)) return 1;
+        } else if (all) {
+                if (allgather_rows(c, xf, c->n_off)) return 1;
+                if (download_rows(c, x, xf, c->N)) return 1;
+        } else if (download_rows(c, x + (size_t)n0 * n, c->n_old2new ? xf : xf + (size_t)n0 * np, ln, c->n_old2new, n0)) return 1;
+        *k = hk;
+        return 0;
+}
+
+int blk_kernel_basis(blk_ctx *c, uint32_t *x, int32_t *k)
+{
+        if (!c || !x || !k) return fail("blk_kernel_basis: null argument");
+        if (c->is_group()) {
+                // every GPU writes its own rows into the one host block
+                std::vector<int32_t> kk(c->members.size(), 0);
+                if (group_run(c, [&](blk_ctx *mem, int r) { return kernel_basis_rank(mem, x, &kk[(size_t)r], false); })) return 1;
+                *k = kk[0];
+                return 0;
+        }
+        return kernel_basis_rank(c, x, k, true);
+}
+
 int blk_get_small(blk_ctx *c, uint32_t *vtAv, uint32_t *vtAAv, uint32_t *winv, uint32_t *d, int32_t *npiv)
 {
         if (!c) return fail("blk_get_small: null context");

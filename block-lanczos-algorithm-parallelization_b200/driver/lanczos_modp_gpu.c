@@ -19,6 +19,9 @@
  *   - checkpoint files are formatted into *.tmp and renamed into place together, with a commit
  *     marker (checkpoint.commit) that --load-checkpoint verifies;
  *   - BLK_GPUS=G in the environment shards the job over G GPUs of the box (same files, same output);
+ *   - --kernel-basis (new, needs --output-file): after the loop, the final Gaussian elimination of block
+ *     Lanczos extracts the independent kernel vectors inside span(v) (blk_kernel_basis); the output file then
+ *     holds those k columns instead of the n columns of v.  Without it the output is the reference's;
  *   - the GPU runs iterations in batches, so progress is reported per batch.
  */
 #define _POSIX_C_SOURCE 200809L
@@ -42,7 +45,7 @@ struct options {
         int n;
         bool right;
         int stop_after;
-        bool checkpoint, resume;
+        bool checkpoint, resume, kernel_basis;
         double checkpoint_every;
         int device;
 };
@@ -67,6 +70,7 @@ static void usage(const char *argv0)
         printf("--stop-after N              stop the algorithm after N iterations\n");
         printf("--checkpoint cp             enable checkpointing every cp seconds [default cp = 60 s]\n");
         printf("--load-checkpoint           load vectors from checkpointing files\n");
+        printf("--kernel-basis              store only independent kernel vectors (needs --output-file)\n");
         printf("\n");
         printf("The --matrix and --prime arguments are required\n");
         printf("The --stop-after and --output-file arguments mutually exclusive\n");
@@ -85,6 +89,7 @@ static void parse_options(struct options *o, int argc, char **argv)
                 {"stop-after", required_argument, NULL, 's'},
                 {"checkpoint", optional_argument, NULL, 'c'},
                 {"load-checkpoint", no_argument, NULL, 'L'},
+                {"kernel-basis", no_argument, NULL, 'K'},
                 {NULL, 0, NULL, 0}};
         memset(o, 0, sizeof(*o));
         o->n = 1;
@@ -111,12 +116,15 @@ static void parse_options(struct options *o, int argc, char **argv)
                                 o->checkpoint_every = atoi(optarg);
                         break;
                 case 'L': o->resume = true; break;
+                case 'K': o->kernel_basis = true; break;
                 default: errx(1, "Unknown option\n");
                 }
         }
         if (!o->matrix || o->prime == 0)
                 usage(argv[0]);
         if (o->output && o->stop_after > 0)
+                usage(argv[0]);
+        if (o->kernel_basis && !o->output)
                 usage(argv[0]);
         if (o->prime > 0x7fffffffull)
                 errx(1, "p is capped at 2**31 - 1.");
@@ -423,7 +431,20 @@ int main(int argc, char **argv)
         }
         printf("  - Terminated in %.1fs after %d iterations\n", wall() - pg.start, n_iterations);
 
-        if (o.output)
+        if (o.output && o.kernel_basis) {
+                /* the kernel vectors inside span(v): k independent columns, checked like checker_modp would */
+                int32_t k = 0, ok = 0;
+                GPU(blk_kernel_basis(ctx, tmp, &k));
+                printf("  - Kernel basis: %d independent vectors\n", (int)k);
+                if (k == 0)
+                        errx(1, "no kernel vector in the final block: nothing to save");
+                GPU(blk_check_kernel_block(ctx, tmp, &ok));
+                printf(ok ? "  - OK: kernel basis * M == 0\n" : "  - KO: kernel basis * M != 0\n");
+                for (long r = 0; r < N; r++)                 /* N x n, stride n -> N x k, stride k */
+                        for (int j = 0; j < k; j++)
+                                Av[r * k + j] = tmp[r * n + j];
+                kernel_block_save(o.output, (int)N, (int)k, Av);
+        } else if (o.output)
                 kernel_block_save(o.output, (int)N, n, v);
         else
                 printf("Not saving result (no --output given)\n");

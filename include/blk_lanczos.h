@@ -143,6 +143,13 @@ int  blk_final_check(blk_ctx *ctx, int32_t *v_nonzero, int32_t *vtm_zero);
 /* The property checker_modp verifies (checker_modp.c:146-204) for a candidate block x of N*n u32:
  * every entry < prime, x not all zero, and x*M == 0 (M*x == 0 for --right).  *ok = 1 if all hold. */
 int  blk_check_kernel_block(blk_ctx *ctx, const uint32_t *x, int32_t *ok);
+/* The kernel vectors inside span(v) (the final Gaussian elimination of block Lanczos, Montgomery 1995; the
+ * reference has no such step, DESIGN.md section 12): with T = M^T v (resp. M v), X = v A where the columns of A
+ * are the standard null basis of T reduced to those that stay independent through v.  x receives N*n u32
+ * (row-major, stride n, host order): columns [0,k) hold X, columns [k,n) are zero; *k = rank([T; v]) - rank(T).
+ * The columns of X are independent, x*M == 0 (M*x == 0 for --right), and they span every such vector in span(v).
+ * Callable at any point of the loop; v, tmp, Av and p are left untouched. */
+int  blk_kernel_basis(blk_ctx *ctx, uint32_t *x, int32_t *k);
 /* n x n results of the last executed iteration (any may be NULL): vtAv, vtAAv,
  * winv are n*n, d is n; *npiv the value semi_inverse returned.            */
 int  blk_get_small(blk_ctx *ctx, uint32_t *vtAv, uint32_t *vtAAv, uint32_t *winv, uint32_t *d,
