@@ -27,9 +27,9 @@ PHASES = ("spmv1", "spmv2", "dots", "small", "ortho", "exchange")
 
 # every symbol include/blk_lanczos.h declares
 ABI_SYMBOLS = (
-    "blk_abi_version", "blk_last_error", "blk_device_count", "blk_nccl_unique_id", "blk_create",
+    "blk_abi_version", "blk_last_error", "blk_device_count", "blk_nccl_unique_id", "blk_create", "blk_create_system",
     "blk_destroy", "blk_plan_shards", "blk_plan_grid", "blk_block_pad", "blk_set_state", "blk_iterate", "blk_get_state", "blk_get_state_local", "blk_final_check",
-    "blk_check_kernel_block", "blk_kernel_basis", "blk_get_small",
+    "blk_check_kernel_block", "blk_kernel_basis", "blk_solve", "blk_get_small",
     "blk_spmv", "blk_block_dot_products", "blk_semi_inverse", "blk_orthogonalize",
     "blk_set_profiling", "blk_get_phase_times", "blk_time_spmv", "blk_kernel_launches", "blk_get_info",
 )
@@ -55,7 +55,7 @@ class blk_info(C.Structure):
         ("local_M0", C.c_int64), ("local_M1", C.c_int64), ("nnz_local", C.c_int64 * 2),
         ("stored_local", C.c_int64 * 2), ("tiles", C.c_int64 * 2), ("n", C.c_int32), ("n_pad", C.c_int32),
         ("chunk_len", C.c_int32 * 2), ("groups_per_warp", C.c_int32), ("device_bytes", C.c_int64),
-        ("loop_mode", C.c_int32), ("reserved", C.c_int32), ("bands", C.c_int32 * 2),
+        ("loop_mode", C.c_int32), ("nrhs", C.c_int32), ("bands", C.c_int32 * 2),
     ]
 
 
@@ -78,6 +78,7 @@ def load_library(path: str | None = None) -> C.CDLL:
     L.blk_device_count.argtypes = [C.POINTER(C.c_int)]
     L.blk_nccl_unique_id.argtypes = [vp]
     L.blk_create.argtypes = [C.POINTER(vp), C.POINTER(blk_params)]
+    L.blk_create_system.argtypes = [C.POINTER(vp), C.POINTER(blk_params), vp, i32, i32]
     L.blk_destroy.argtypes = [vp]
     L.blk_plan_shards.argtypes = [vp, i64, i64, i32, vp]
     L.blk_plan_grid.argtypes = [vp, vp, i64, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp]
@@ -90,6 +91,7 @@ def load_library(path: str | None = None) -> C.CDLL:
     L.blk_final_check.argtypes = [vp, C.POINTER(i32), C.POINTER(i32)]
     L.blk_check_kernel_block.argtypes = [vp, vp, C.POINTER(i32)]
     L.blk_kernel_basis.argtypes = [vp, vp, C.POINTER(i32)]
+    L.blk_solve.argtypes = [vp, vp, vp]
     L.blk_get_small.argtypes = [vp, vp, vp, vp, vp, C.POINTER(i32)]
     L.blk_spmv.argtypes = [vp, vp, vp, i32]
     L.blk_block_dot_products.argtypes = [vp, vp, vp, i64, vp, vp]
@@ -171,10 +173,16 @@ class BlockLanczos:
 
     def __init__(self, M=None, *, n: int, prime: int, right: bool = False, device: int = 0,
                  rank: int = 0, world: int = 1, nccl_id: bytes | None = None, stream: int | None = None,
-                 chunk_len: int = 0, use_graph: int = -1, device_coo=None):
+                 chunk_len: int = 0, use_graph: int = -1, device_coo=None, rhs=None, rhs_device=None):
         """`M` is a host SparseCOO; alternatively `device_coo=(nrows, ncols, nnz, i_ptr, j_ptr, x_ptr)`
         gives raw CUDA device pointers (int32, int32, uint32) on `device`.  `rank=BLK_RANK_ALL` with
-        `world=W` makes ONE context drive W GPUs (devices device..device+W-1) from this process."""
+        `world=W` makes ONE context drive W GPUs (devices device..device+W-1) from this process.
+
+        `rhs` (an Mc x r integer array, 1 <= r <= n; Mc = nrows for --right, ncols for --left) makes the context of
+        the system M x = b (x M = b for --left), blk_create_system: the loop then runs on the augmented matrix, so
+        `nrows` / `ncols` / `N` / `pad` are its sizes; `N0` is the original length and `nrhs` = r.  Negative
+        entries are taken like the MatrixMarket loader takes them (-k is 2^32 - k before the reduction mod p).
+        `rhs_device=(ptr, r)` gives that block instead as a raw CUDA device pointer (uint32, Mc x r) on `device`."""
         self.L = load_library()
         self.n, self.prime, self.right = int(n), int(prime), bool(right)
         prm = blk_params()
@@ -192,6 +200,20 @@ class BlockLanczos:
             prm.nrows, prm.ncols, prm.nnz = M.nrows, M.ncols, M.nnz
             prm.Mi, prm.Mj, prm.Mx = mi.ctypes.data, mj.ctypes.data, mx.ctypes.data
         self.nrows, self.ncols, self.nnz = int(prm.nrows), int(prm.ncols), int(prm.nnz)
+        self.nrhs = 0
+        b_ptr, b_dev = None, 0
+        if rhs_device is not None:
+            b_ptr, b_dev, self.nrhs = C.c_void_p(rhs_device[0]), 1, int(rhs_device[1])
+        elif rhs is not None:
+            b = np.asarray(rhs)
+            if b.ndim == 1:
+                b = b.reshape(-1, 1)
+            if b.ndim != 2 or b.shape[0] != (self.nrows if right else self.ncols):
+                raise BlkError(f"rhs must be an Mc x r array (Mc = {self.nrows if right else self.ncols}), "
+                               f"got shape {b.shape}")
+            b = _u32(b.astype(np.int64) % (1 << 32) if b.dtype.kind == "i" else b)
+            keep.append(b)
+            b_ptr, self.nrhs = _ptr(b), int(b.shape[1])
         prm.n, prm.prime, prm.right_kernel, prm.device = n, prime, int(right), device
         prm.rank, prm.world = rank, world
         idbuf = None
@@ -201,11 +223,19 @@ class BlockLanczos:
         prm.stream = stream
         prm.chunk_len, prm.use_graph = chunk_len, use_graph
         h = C.c_void_p()
-        rc = self.L.blk_create(C.byref(h), C.byref(prm))
+        if self.nrhs:
+            rc = self.L.blk_create_system(C.byref(h), C.byref(prm), b_ptr, self.nrhs, b_dev)
+        else:
+            rc = self.L.blk_create(C.byref(h), C.byref(prm))
         del keep, idbuf
         if rc:
             raise BlkError(self.L.blk_last_error().decode())
         self.h = h
+        self.N0 = self.ncols if right else self.nrows
+        if right:
+            self.ncols += self.nrhs
+        else:
+            self.nrows += self.nrhs
         self.N = self.ncols if right else self.nrows
         self.Mc = self.nrows if right else self.ncols
         self.pad = block_pad(self.nrows, self.ncols, n, right)
@@ -314,6 +344,17 @@ class BlockLanczos:
         k = C.c_int32(0)
         self._ck(self.L.blk_kernel_basis(self.h, _ptr(x), C.byref(k)))
         return x.reshape(self.N, self.n)[:, :k.value].copy()
+
+    def solve(self):
+        """The solutions inside span(v) of a context made with `rhs` (blk_solve): (x, found), x an N0 x r uint32
+        array, found a bool array of r flags.  M x[:, j] == b_j (x[:, j]^T M == b_j for --left) for every found j;
+        the other columns are zero (no solution in span(v): the system may be inconsistent)."""
+        if not self.nrhs:
+            raise BlkError("solve() needs a context created with rhs=")
+        x = np.empty(self.N0 * self.nrhs, dtype=np.uint32)
+        found = np.zeros(self.nrhs, dtype=np.int32)
+        self._ck(self.L.blk_solve(self.h, _ptr(x), _ptr(found)))
+        return x.reshape(self.N0, self.nrhs), found.astype(bool)
 
     def get_small(self):
         n = self.n

@@ -300,3 +300,28 @@ int launch_kb_reduce(int np, const KbArgs &a, cudaStream_t st);
 int launch_kb_small(int np, const KbArgs &a, cudaStream_t st);
 // k_kb_apply: x = v A
 int launch_kb_apply(int np, const KbArgs &a, cudaStream_t st);
+// solve.cu: inhomogeneous systems (blk_create_system, blk_solve), DESIGN.md section 13.
+// The non-zeros of -B (Mc x r, row-major, device) as COO triplets of the augmented matrix: (i, N + j) for --right,
+// (N + j, i) for --left.  *count receives their number; with Mi == nullptr nothing is written (a first call sizes the
+// buffers, a second one fills them).  Returns an error message or "".
+std::string rhs_triplets(const u32 *B, int64_t Mc, int r, int64_t N, int right, u32 p, int32_t *Mi, int32_t *Mj, u32 *Mx,
+                         int64_t *count, cudaStream_t st);
+int pad_width(int w);                // smallest power of two >= w
+struct SolveArgs {
+        int np = 1, r = 1, rp = 1;     // n_pad, right-hand sides, r padded to a power of two (<= n_pad)
+        ModP m;
+        const u32 *A = nullptr;        // n_pad x n_pad: A_S of k_kb_small
+        const int *k = nullptr;        // its number of columns
+        u32 *tail = nullptr;           // r x n_pad: the tail rows of v (rows N .. N+r-1 of the augmented problem)
+        u32 *W = nullptr;              // n_pad x rp: W = A_S C
+        int *found = nullptr;          // [r]
+        const u32 *v = nullptr;        // this rank's rows of v (vrows x n_pad)
+        int64_t vrows = 0;
+        u32 *x = nullptr;              // vrows x rp: x = v W
+};
+// k_solve_tail: the tail rows this rank owns (device rows [n0, n1) of the full-length v_full), zero elsewhere
+int launch_solve_tail(const SolveArgs &a, int64_t N0, const u32 *v_full, const u32 *map, int64_t n0, int64_t n1, cudaStream_t st);
+// k_solve_small: tail, A, k -> W, found
+int launch_solve_small(const SolveArgs &a, cudaStream_t st);
+// k_solve_apply: x = v W
+int launch_solve_apply(const SolveArgs &a, cudaStream_t st);

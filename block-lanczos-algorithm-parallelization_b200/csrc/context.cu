@@ -101,6 +101,7 @@ struct blk_ctx {
         int device = 0, rank = 0, world = 1, right = 0;
         int32_t nrows = 0, ncols = 0;
         int64_t N = 0, Mc = 0;
+        int nrhs = 0;                           // blk_create_system: right-hand sides appended to M (N counts them too)
         std::vector<int64_t> n_off, m_off;      // row partition of the N and Mc dimensions
         SpOp S1, S2;                            // tmp <- S1 v ; Av <- S2 tmp
         u32 *v = nullptr, *tmp = nullptr;       // full length: N*np, Mc*np
@@ -481,18 +482,20 @@ int scan_rows(blk_ctx *c, const u32 *a, int64_t rows, int *any_nonzero, int *any
         return 0;
 }
 
-// buf holds gather_cap(off) rows; every rank contributes rows [off[rank], off[rank+1]) in place
-int allgather_rows(blk_ctx *c, u32 *buf, const std::vector<int64_t> &off)
+// buf holds gather_cap(off) rows; every rank contributes rows [off[rank], off[rank+1]) in place.
+// wp: words per row (0: n_pad)
+int allgather_rows(blk_ctx *c, u32 *buf, const std::vector<int64_t> &off, int wp = 0)
 {
+        const int np = wp ? wp : c->geo.np;
         if (c->nccl_allgather && equal_blocks(off)) {
-                size_t cnt = (size_t)(off[1] - off[0]) * c->geo.np;
+                size_t cnt = (size_t)(off[1] - off[0]) * np;
                 NC(c->nccl_allgather(buf + (size_t)c->rank * cnt, buf, cnt, ncclUint32, c->comm, c->stream));
                 return 0;
         }
         NC(g_nccl.GroupStart());
         for (int r = 0; r < c->world; r++) {
-                size_t cnt = (size_t)(off[r + 1] - off[r]) * c->geo.np;
-                u32 *ptr = buf + (size_t)off[r] * c->geo.np;
+                size_t cnt = (size_t)(off[r + 1] - off[r]) * np;
+                u32 *ptr = buf + (size_t)off[r] * np;
                 if (cnt) NC(g_nccl.Broadcast(ptr, ptr, cnt, ncclUint32, r, c->comm, c->stream));
         }
         NC(g_nccl.GroupEnd());
@@ -1104,10 +1107,12 @@ int upload_rows(blk_ctx *c, u32 *dst, const u32 *src_host, int64_t rows, const u
         CU(cudaStreamSynchronize(c->stream));
         return 0;
 }
-// `map` (device, nullable): host row r0 + r comes from device row map[r0 + r] of `src` (else row r of `src`)
-int download_rows(blk_ctx *c, u32 *dst_host, const u32 *src, int64_t rows, const u32 *map = nullptr, int64_t r0 = 0)
+// `map` (device, nullable): host row r0 + r comes from device row map[r0 + r] of `src` (else row r of `src`).
+// w / wp: words per host / device row (0: n / n_pad)
+int download_rows(blk_ctx *c, u32 *dst_host, const u32 *src, int64_t rows, const u32 *map = nullptr, int64_t r0 = 0,
+                  int w = 0, int wp = 0)
 {
-        const int n = c->geo.n, np = c->geo.np;
+        const int n = w ? w : c->geo.n, np = wp ? wp : c->geo.np;
         if (rows == 0) return 0;
         if (n == np && !map) {
                 CU(cudaMemcpyAsync(dst_host, src, sizeof(u32) * (size_t)rows * n, cudaMemcpyDeviceToHost, c->stream));
@@ -2073,10 +2078,88 @@ int blk_create(blk_ctx **out, const blk_params *prm)
 }
 
 
+// blk_create_system: the COO of M and the non-zeros of -B (rhs_triplets) in one device COO, handed to blk_create as
+// the augmented matrix [M | -B] (--right) or [M ; -B^T] (--left)
+static int create_system(blk_ctx **out, const blk_params *prm, const uint32_t *B, int32_t nrhs, int32_t b_on_device)
+{
+        if (!out) return fail("blk_create_system: null output pointer");
+        *out = nullptr;
+        if (!prm || prm->abi_version != BLK_ABI_VERSION) return fail("blk_params.abi_version mismatch");
+        if (prm->n < 1 || prm->n > BLK_MAX_N) return fail("blocking factor n must be in [1,64]");
+        if (prm->nrows < 1 || prm->ncols < 1 || prm->nnz < 0) return fail("bad matrix dimensions");
+        if (prm->nnz > 0 && (!prm->Mi || !prm->Mj || !prm->Mx)) return fail("null COO arrays");
+        if (nrhs < 1 || nrhs > prm->n) return fail("blk_create_system: the number of right-hand sides must be in [1, n]");
+        if (!B) return fail("blk_create_system: null right-hand-side block");
+        ModP m;
+        if (!modp_make(&m, prm->prime)) return fail("prime must satisfy 2 <= p < 2^31");
+        const int right = prm->right_kernel ? 1 : 0;
+        const int64_t N = right ? prm->ncols : prm->nrows, Mc = right ? prm->nrows : prm->ncols;
+        if (N + nrhs > INT32_MAX) return fail("blk_create_system: the matrix is too large for the appended right-hand sides");
+        int ndev = 0;
+        cudaError_t e0 = cudaGetDeviceCount(&ndev);
+        if (e0 != cudaSuccess || ndev == 0)
+                return fail(std::string("no CUDA device (there is no CPU fallback): ") + cudaGetErrorString(e0));
+        if (prm->device < 0 || prm->device >= ndev) return fail("device ordinal out of range");
+        CU(cudaSetDevice(prm->device));
+        struct Bufs {
+                std::vector<void *> p;
+                cudaStream_t st = nullptr;
+                ~Bufs() { for (void *q : p) cudaFree(q); if (st) cudaStreamDestroy(st); }
+        } bufs;
+        auto grab = [&](void **dst, size_t bytes) {
+                cudaError_t e = cudaMalloc(dst, bytes ? bytes : 4);
+                if (e == cudaSuccess) bufs.p.push_back(*dst);
+                return e;
+        };
+        CU(cudaStreamCreateWithFlags(&bufs.st, cudaStreamNonBlocking));
+        const cudaStream_t st = bufs.st;
+        const u32 *dB = B;
+        if (!b_on_device) {
+                u32 *hb = nullptr;
+                CU(grab((void **)&hb, sizeof(u32) * (size_t)Mc * nrhs));
+                CU(cudaMemcpyAsync(hb, B, sizeof(u32) * (size_t)Mc * nrhs, cudaMemcpyHostToDevice, st));
+                dB = hb;
+        }
+        int64_t add = 0, added = 0;
+        std::string err = rhs_triplets(dB, Mc, nrhs, N, right, m.p, nullptr, nullptr, nullptr, &add, st);
+        if (!err.empty()) return fail(err);
+        const int64_t nnz = prm->nnz, tot = nnz + add;
+        int32_t *di = nullptr, *dj = nullptr;
+        u32 *dx = nullptr;
+        CU(grab((void **)&di, sizeof(int32_t) * (size_t)tot));
+        CU(grab((void **)&dj, sizeof(int32_t) * (size_t)tot));
+        CU(grab((void **)&dx, sizeof(u32) * (size_t)tot));
+        if (nnz) {
+                const cudaMemcpyKind kind = prm->coo_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+                CU(cudaMemcpyAsync(di, prm->Mi, sizeof(int32_t) * (size_t)nnz, kind, st));
+                CU(cudaMemcpyAsync(dj, prm->Mj, sizeof(int32_t) * (size_t)nnz, kind, st));
+                CU(cudaMemcpyAsync(dx, prm->Mx, sizeof(u32) * (size_t)nnz, kind, st));
+        }
+        err = rhs_triplets(dB, Mc, nrhs, N, right, m.p, di + nnz, dj + nnz, dx + nnz, &added, st);
+        if (!err.empty()) return fail(err);
+        if (added != add) return fail("blk_create_system: right-hand-side count mismatch");
+        CU(cudaStreamSynchronize(st));
+        blk_params p2 = *prm;
+        if (right) p2.ncols += nrhs;
+        else p2.nrows += nrhs;
+        p2.nnz = tot; p2.Mi = di; p2.Mj = dj; p2.Mx = dx; p2.coo_on_device = 1;
+        if (blk_create(out, &p2)) return 1;
+        blk_ctx *c = *out;
+        c->nrhs = nrhs;
+        for (blk_ctx *mem : c->members) mem->nrhs = nrhs;
+        return 0;
+}
+
+
 // ---------------------------------------------------------------------------------- C ABI
 extern "C" {
 
 int blk_abi_version(void) { return BLK_ABI_VERSION; }
+
+int blk_create_system(blk_ctx **out, const blk_params *prm, const uint32_t *B, int32_t nrhs, int32_t b_on_device)
+{
+        return create_system(out, prm, B, nrhs, b_on_device);
+}
 
 const char *blk_last_error(void) { return g_err.c_str(); }
 
@@ -2615,6 +2698,100 @@ int blk_kernel_basis(blk_ctx *c, uint32_t *x, int32_t *k)
         return kernel_basis_rank(c, x, k, true);
 }
 
+// One rank of blk_solve: A_S and k exactly as kernel_basis_rank obtains them, the r tail rows of v from their owners
+// (one NCCL all-reduce: every entry has one owner, the others add zero), the r x k stage redundantly on every rank,
+// and x = v W for the rows this rank owns.  whole: as in kernel_basis_rank.  Rows from N0 = N - r on (the
+// right-hand-side coordinates) are not part of x.
+static int solve_rank(blk_ctx *c, uint32_t *x, int32_t *found, bool whole)
+{
+        CU(cudaSetDevice(c->device));
+        const int n = c->geo.n, np = c->geo.np, r = c->nrhs, rp = pad_width(r);
+        if (c->grid_on && grid_export(c)) return 1;
+        const int64_t n0 = c->n0(), ln = c->n1() - n0, lm = c->m1() - c->m0(), N0 = c->N - r;
+        bool have = c->tmp_is_spmv || (c->mg_recur && c->ran_since_set);
+        const size_t rec_words = (size_t)(n + 1) * np;
+        KbArgs a;
+        a.n = n; a.world = c->world; a.m = c->m;
+        a.v = c->v + (size_t)n0 * np; a.vrows = ln;
+        a.t = c->tmp + (size_t)c->m0() * np; a.trows = lm;
+        a.ctas = kb_ctas(std::max(ln, lm));
+        struct Bufs {
+                std::vector<void *> p;
+                ~Bufs() { for (void *q : p) cudaFree(q); }
+        } bufs;
+        auto grab = [&](void **dst, size_t bytes) {
+                cudaError_t e = cudaMalloc(dst, bytes ? bytes : 4);
+                if (e == cudaSuccess) bufs.p.push_back(*dst);
+                return e;
+        };
+        u32 *scratch = nullptr, *xf = nullptr;
+        if (!have) {
+                if (c->world > 1 && allgather_rows(c, c->v, c->n_off)) return 1;
+                CU(grab((void **)&scratch, sizeof(u32) * (size_t)lm * np));
+                c->launches += launch_spmv(c->S1, c->geo, c->m, c->v, scratch, nullptr, c->stream);
+                a.t = scratch;
+        }
+        CU(grab((void **)&a.part, sizeof(u32) * (size_t)2 * a.ctas * n * np));
+        CU(grab((void **)&a.prank, sizeof(int) * (size_t)2 * a.ctas));
+        CU(grab((void **)&a.counter, sizeof(unsigned)));
+        CU(grab((void **)&a.rec_all, sizeof(u32) * (size_t)c->world * 2 * rec_words));
+        CU(grab((void **)&a.A, sizeof(u32) * (size_t)np * np));
+        CU(grab((void **)&a.k, sizeof(int)));
+        a.rec_own = a.rec_all + (size_t)c->rank * 2 * rec_words;
+        SolveArgs s;
+        s.np = np; s.r = r; s.rp = rp; s.m = c->m; s.A = a.A; s.k = a.k;
+        s.v = a.v; s.vrows = ln;
+        CU(grab((void **)&s.tail, sizeof(u32) * (size_t)r * np));
+        CU(grab((void **)&s.W, sizeof(u32) * (size_t)np * rp));
+        CU(grab((void **)&s.found, sizeof(int) * (size_t)r));
+        CU(grab((void **)&xf, sizeof(u32) * (size_t)gather_cap(c->n_off) * rp));
+        s.x = xf + (size_t)n0 * rp;
+        CU(cudaMemsetAsync(a.counter, 0, sizeof(unsigned), c->stream));
+        c->launches += launch_kb_reduce(np, a, c->stream);
+        if (c->world > 1)
+                NC(g_nccl.AllGather(a.rec_own, a.rec_all, 2 * rec_words, ncclUint32, c->comm, c->stream));
+        c->launches += launch_kb_small(np, a, c->stream);
+        c->launches += launch_solve_tail(s, N0, c->v, c->n_old2new, n0, n0 + ln, c->stream);
+        if (c->world > 1)
+                NC(g_nccl.AllReduce(s.tail, s.tail, (size_t)r * np, ncclUint32, ncclSum, c->comm, c->stream));
+        c->launches += launch_solve_small(s, c->stream);
+        c->launches += launch_solve_apply(s, c->stream);
+        std::vector<int> hf((size_t)r, 0);
+        CU(cudaMemcpyAsync(hf.data(), s.found, sizeof(int) * (size_t)r, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        CU(cudaGetLastError());
+        // down to the host like X in kernel_basis_rank, host rows [0, N0) only
+        const bool all = whole && c->world > 1;
+        if (c->relabel_mg()) {
+                const int64_t r0 = all ? 0 : std::min(c->h0(), N0), r1 = all ? N0 : std::min(c->h1(), N0);
+                if (allgather_rows(c, xf, c->n_off, rp)) return 1;
+                if (download_rows(c, x + (size_t)r0 * r, xf, r1 - r0, c->n_old2new, r0, r, rp)) return 1;
+        } else if (all) {
+                if (allgather_rows(c, xf, c->n_off, rp)) return 1;
+                if (download_rows(c, x, xf, N0, nullptr, 0, r, rp)) return 1;
+        } else {
+                const int64_t lo = std::min(n0, N0), hi = std::min(n0 + ln, N0);
+                if (download_rows(c, x + (size_t)lo * r, c->n_old2new ? xf : xf + (size_t)lo * rp, hi - lo, c->n_old2new, lo, r, rp))
+                        return 1;
+        }
+        for (int j = 0; j < r; j++) found[j] = hf[(size_t)j];
+        return 0;
+}
+
+int blk_solve(blk_ctx *c, uint32_t *x, int32_t *found)
+{
+        if (!c || !x || !found) return fail("blk_solve: null argument");
+        if (c->nrhs < 1) return fail("blk_solve: the context has no right-hand sides (create it with blk_create_system)");
+        if (c->is_group()) {
+                // every GPU writes its own rows into the one host block
+                std::vector<std::vector<int32_t>> ff(c->members.size(), std::vector<int32_t>((size_t)c->nrhs, 0));
+                if (group_run(c, [&](blk_ctx *mem, int r) { return solve_rank(mem, x, ff[(size_t)r].data(), false); })) return 1;
+                for (int j = 0; j < c->nrhs; j++) found[j] = ff[0][(size_t)j];
+                return 0;
+        }
+        return solve_rank(c, x, found, true);
+}
+
 int blk_get_small(blk_ctx *c, uint32_t *vtAv, uint32_t *vtAAv, uint32_t *winv, uint32_t *d, int32_t *npiv)
 {
         if (!c) return fail("blk_get_small: null context");
@@ -2868,6 +3045,7 @@ int blk_get_info(blk_ctx *c, blk_info *info)
         }
         memset(info, 0, sizeof(*info));
         info->N = c->N; info->Mc = c->Mc;
+        info->nrhs = c->nrhs;
         // (with relabelled rows on several GPUs: the HOST rows this rank moves in blk_set_state / blk_get_state_local)
         info->local_N0 = c->h0(); info->local_N1 = c->h1();
         info->local_M0 = c->m0(); info->local_M1 = c->m1();

@@ -12,6 +12,7 @@
  *
  * USAGE:
  *      $ ./lanczos_modp --prime 65537 --n 4 --matrix random_small.mtx
+ *      $ ./lanczos_modp --prime 65537 --n 16 --matrix M.mtx --rhs B.mtx --output-file X.mtx [--right]
  *
  * Deviations from the reference, all documented in DESIGN.md:
  *   - p may be as large as 2^31-1 (the reference stops at 2^30-35);
@@ -22,6 +23,10 @@
  *   - --kernel-basis (new, needs --output-file): after the loop, the final Gaussian elimination of block
  *     Lanczos extracts the independent kernel vectors inside span(v) (blk_kernel_basis); the output file then
  *     holds those k columns instead of the n columns of v.  Without it the output is the reference's;
+ *   - --rhs FILE (new, needs --output-file): solve M*X = B (--right) or X*M = B (--left) for the r <= n columns
+ *     of the MatrixMarket array B (Mc x r, the format of the output file).  The loop runs on the augmented
+ *     matrix [M | -B] (resp. [M ; -B^T]); blk_solve then extracts the solutions and the output file holds the
+ *     N x r block X.  Exit status 1 and no file when some right-hand side is not solved;
  *   - the GPU runs iterations in batches, so progress is reported per batch.
  */
 #define _POSIX_C_SOURCE 200809L
@@ -46,6 +51,7 @@ struct options {
         bool right;
         int stop_after;
         bool checkpoint, resume, kernel_basis;
+        const char *rhs;
         double checkpoint_every;
         int device;
 };
@@ -71,6 +77,7 @@ static void usage(const char *argv0)
         printf("--checkpoint cp             enable checkpointing every cp seconds [default cp = 60 s]\n");
         printf("--load-checkpoint           load vectors from checkpointing files\n");
         printf("--kernel-basis              store only independent kernel vectors (needs --output-file)\n");
+        printf("--rhs FILENAME              solve M*X = B (X*M = B with --left) for the array B (needs --output-file)\n");
         printf("\n");
         printf("The --matrix and --prime arguments are required\n");
         printf("The --stop-after and --output-file arguments mutually exclusive\n");
@@ -90,6 +97,7 @@ static void parse_options(struct options *o, int argc, char **argv)
                 {"checkpoint", optional_argument, NULL, 'c'},
                 {"load-checkpoint", no_argument, NULL, 'L'},
                 {"kernel-basis", no_argument, NULL, 'K'},
+                {"rhs", required_argument, NULL, 'B'},
                 {NULL, 0, NULL, 0}};
         memset(o, 0, sizeof(*o));
         o->n = 1;
@@ -117,11 +125,18 @@ static void parse_options(struct options *o, int argc, char **argv)
                         break;
                 case 'L': o->resume = true; break;
                 case 'K': o->kernel_basis = true; break;
+                case 'B': o->rhs = optarg; break;
                 default: errx(1, "Unknown option\n");
                 }
         }
         if (!o->matrix || o->prime == 0)
                 usage(argv[0]);
+        if (o->rhs) {
+                if (!o->output)
+                        errx(1, "usage: --rhs needs --output-file");
+                if (o->kernel_basis || o->stop_after > 0 || o->checkpoint || o->resume)
+                        errx(1, "usage: --rhs cannot be combined with --kernel-basis, --stop-after, --checkpoint or --load-checkpoint");
+        }
         if (o->output && o->stop_after > 0)
                 usage(argv[0]);
         if (o->kernel_basis && !o->output)
@@ -334,9 +349,23 @@ int main(int argc, char **argv)
         mtx_load(&M, o.matrix, o.prime);
 
         const int n = o.n;
-        const long N = o.right ? M.ncols : M.nrows;          /* length of the Lanczos vectors */
-        const long Mc = o.right ? M.nrows : M.ncols;
-        const long pad = (long)blk_block_pad(M.nrows, M.ncols, n, o.right);
+        /* --rhs: the Mc x r block B; the Lanczos vectors of the augmented matrix have N + r rows */
+        int nrhs = 0;
+        uint32_t *B = NULL;
+        if (o.rhs) {
+                int brows = 0;
+                B = mtx_load_array(o.rhs, o.prime, &brows, &nrhs);
+                const long want = o.right ? M.nrows : M.ncols;
+                if (brows != want)
+                        errx(1, "%s has %d rows, expected %ld (%s of the matrix)", o.rhs, brows, want, o.right ? "rows" : "columns");
+                if (nrhs > n)
+                        errx(1, "%s has %d right-hand sides, more than the blocking factor n = %d", o.rhs, nrhs, n);
+        }
+        const int anrows = M.nrows + (o.right ? 0 : nrhs), ancols = M.ncols + (o.right ? nrhs : 0);
+        const long N = o.right ? ancols : anrows;            /* length of the Lanczos vectors */
+        const long Mc = o.right ? anrows : ancols;
+        const long N0 = N - nrhs;                            /* the unknowns of the system */
+        const long pad = (long)blk_block_pad(anrows, ancols, n, o.right);
 
         printf("Block Lanczos\n");
         char hs[16];
@@ -361,7 +390,11 @@ int main(int argc, char **argv)
         prm.world = gpus; prm.rank = gpus > 1 ? BLK_RANK_ALL : 0;
         blk_ctx *ctx = NULL;
         double t_build = wall();
-        GPU(blk_create(&ctx, &prm));
+        if (o.rhs)
+                GPU(blk_create_system(&ctx, &prm, B, nrhs, 0));
+        else
+                GPU(blk_create(&ctx, &prm));
+        free(B);
         if (gpus > 1)
                 printf("  - Matrix resident on GPUs %d-%d (row blocks) in %.2fs\n", o.device, o.device + gpus - 1, wall() - t_build);
         else
@@ -431,7 +464,46 @@ int main(int argc, char **argv)
         }
         printf("  - Terminated in %.1fs after %d iterations\n", wall() - pg.start, n_iterations);
 
-        if (o.output && o.kernel_basis) {
+        if (o.output && o.rhs) {
+                /* the solutions inside span(v), checked on the device as the kernel block (x_j ; e_j) of the
+                 * augmented matrix */
+                uint32_t *x = calloc((size_t)N0 * (size_t)nrhs, sizeof(*x));
+                int32_t *found = calloc((size_t)nrhs, sizeof(*found));
+                if (!x || !found)
+                        errx(1, "cannot allocate the solution block");
+                GPU(blk_solve(ctx, x, found));
+                int solved = 0;
+                for (int j = 0; j < nrhs; j++)
+                        solved += found[j] != 0;
+                printf("  - Solve: %d of %d right-hand sides solved\n", solved, nrhs);
+                if (solved > 0) {
+                        int32_t ok = 0;
+                        memset(tmp, 0, sizeof(*tmp) * (size_t)pad);      /* (N + r) x n, stride n */
+                        for (int j = 0; j < nrhs; j++) {
+                                if (!found[j])
+                                        continue;
+                                for (long r = 0; r < N0; r++)
+                                        tmp[r * n + j] = x[r * nrhs + j];
+                                tmp[(N0 + j) * n + j] = 1;
+                        }
+                        GPU(blk_check_kernel_block(ctx, tmp, &ok));
+                        if (o.right)
+                                printf(ok ? "  - OK: M*X == B\n" : "  - KO: M*X != B\n");
+                        else
+                                printf(ok ? "  - OK: X*M == B\n" : "  - KO: X*M != B\n");
+                }
+                if (solved < nrhs) {
+                        char list[256] = "";
+                        size_t at = 0;
+                        for (int j = 0; j < nrhs && at < sizeof(list) - 16; j++)
+                                if (!found[j])
+                                        at += (size_t)snprintf(list + at, sizeof(list) - at, "%s%d", at ? ", " : "", j + 1);
+                        errx(1, "no solution in the final block for right-hand side(s) %s: the system may be inconsistent, "
+                                "or the block did not reach a solution; nothing saved", list);
+                }
+                kernel_block_save(o.output, (int)N0, nrhs, x);
+                free(x); free(found);
+        } else if (o.output && o.kernel_basis) {
                 /* the kernel vectors inside span(v): k independent columns, checked like checker_modp would */
                 int32_t k = 0, ok = 0;
                 GPU(blk_kernel_basis(ctx, tmp, &k));

@@ -244,6 +244,57 @@ void mtx_load(struct coo_matrix *M, const char *filename, uint64_t prime)
         M->i = Mi; M->j = Mj; M->x = Mx;
 }
 
+uint32_t *mtx_load_array(const char *filename, uint64_t prime, int *rows, int *cols)
+{
+        size_t len, pos = 0, ll;
+        char *buf = slurp(filename, &len);
+        const char *line = next_line(buf, len, &pos, &ll);
+        char banner[16] = "", object[64] = "", format[64] = "", field[64] = "", symm[64] = "";
+        char first[512];
+        if (!line)
+                errx(1, "%s: could not process Matrix Market banner", filename);
+        snprintf(first, sizeof(first), "%.*s", (int)(ll < 500 ? ll : 500), line);
+        if (sscanf(first, "%15s %63s %63s %63s %63s", banner, object, format, field, symm) != 5 ||
+            strcmp(banner, "%%MatrixMarket") != 0)
+                errx(1, "%s: could not process Matrix Market banner", filename);
+        if (!ieq(object, "matrix") || !ieq(format, "array") || !ieq(field, "integer") || !ieq(symm, "general"))
+                errx(1, "%s: [%s %s %s %s] not supported (only matrix array integer general)", filename, object, format,
+                     field, symm);
+        long long nr = 0, nc = 0;
+        for (;;) {
+                line = next_line(buf, len, &pos, &ll);
+                if (!line)
+                        errx(1, "%s: cannot read the array size", filename);
+                if (ll == 0 || line[0] == '%')
+                        continue;
+                const char *p = line, *e = line + ll;
+                if (!scan_int(&p, e, &nr) || !scan_int(&p, e, &nc))
+                        errx(1, "%s: cannot read the array size", filename);
+                break;
+        }
+        if (nr <= 0 || nc <= 0 || nr > 0x7fffffff || nc > 0x7fffffff)
+                errx(1, "%s: bad array size %lld x %lld", filename, nr, nc);
+        uint32_t *x = malloc(sizeof(uint32_t) * (size_t)nr * (size_t)nc);
+        if (!x)
+                err(1, "cannot allocate %lld x %lld values for %s", nr, nc, filename);
+        const char *p = buf + pos, *end = buf + len;
+        long long val;
+        for (long long col = 0; col < nc; col++)            /* column-major, like kernel_block_save */
+                for (long long r = 0; r < nr; r++) {
+                        if (!scan_int(&p, end, &val))
+                                errx(1, "%s: expected %lld values, found fewer", filename, nr * nc);
+                        x[r * nc + col] = (uint32_t)((uint64_t)(uint32_t)(int)val % prime);
+                }
+        while (p < end && is_space(*p))
+                p++;
+        if (p < end)
+                errx(1, "%s: unexpected text after %lld values", filename, nr * nc);
+        free(buf);
+        *rows = (int)nr;
+        *cols = (int)nc;
+        return x;
+}
+
 void mtx_free(struct coo_matrix *M)
 {
         free(M->i); free(M->j); free(M->x);

@@ -22,6 +22,11 @@ struct coo_matrix {
 void mtx_load(struct coo_matrix *M, const char *filename, uint64_t prime);
 void mtx_free(struct coo_matrix *M);
 
+/* dense "array integer general" block of rows x cols (the format kernel_block_save writes, column-major values),
+ * returned row-major (rows x cols, malloc'ed), values reduced mod prime with mtx_load's semantics (-k is 2^32 - k).
+ * errx(1, ...) on any failure. */
+uint32_t *mtx_load_array(const char *filename, uint64_t prime, int *rows, int *cols);
+
 /* kernel block, save_vector_block format (sequential/lanczos_modp.c:673-686):
  * dense "array integer general", "N n", then column-major "%d\n" */
 void kernel_block_save(const char *filename, int nrows, int n, const uint32_t *v);

@@ -80,6 +80,13 @@ int  blk_nccl_unique_id(void *id_out /* BLK_NCCL_ID_BYTES */);
 /* Builds the GPU-resident sparse layouts of M and M^T once from the COO arrays and
  * allocates the four vector blocks v, tmp, Av, p (block_lanczos :592-607), zeroed. */
 int  blk_create(blk_ctx **out, const blk_params *prm);
+/* An inhomogeneous system M*x = b (--right) or x*M = b (--left) for nrhs right-hand sides (DESIGN.md section 13).
+ * B holds Mc*nrhs u32, row-major (row i = the coordinate i of the other dimension, column j = right-hand side j),
+ * reduced mod prime on ingest; it is a host pointer, or a device pointer on prm->device when b_on_device != 0.
+ * 1 <= nrhs <= n.  The context is blk_create's for the augmented matrix [M | -B] (--right) or [M ; -B^T] (--left):
+ * every other entry point works on it, the Lanczos vectors have N + nrhs rows (blk_block_pad, blk_get_info().N),
+ * the last nrhs of them the coordinates of the right-hand sides.  rank / world / BLK_RANK_ALL as for blk_create. */
+int  blk_create_system(blk_ctx **out, const blk_params *prm, const uint32_t *B, int32_t nrhs, int32_t b_on_device);
 int  blk_destroy(blk_ctx *ctx);
 
 /* Host-only: the contiguous, weight-balanced row partition blk_create uses for a `world`-GPU job.
@@ -150,6 +157,12 @@ int  blk_check_kernel_block(blk_ctx *ctx, const uint32_t *x, int32_t *ok);
  * The columns of X are independent, x*M == 0 (M*x == 0 for --right), and they span every such vector in span(v).
  * Callable at any point of the loop; v, tmp, Av and p are left untouched. */
 int  blk_kernel_basis(blk_ctx *ctx, uint32_t *x, int32_t *k);
+/* The solutions inside span(v) of a context made by blk_create_system (fails on any other context).  x receives
+ * N*nrhs u32 (the original N, row-major, stride nrhs, host order), found[nrhs] the flags: column j satisfies
+ * M*x_j == b_j (x_j*M == b_j for --left) when found[j] = 1 and is zero otherwise.  found[j] = 0 means no solution
+ * lies in span(v): the system may be inconsistent, or the block did not reach one.  Callable at any point of the
+ * loop; v, tmp, Av and p are left untouched. */
+int  blk_solve(blk_ctx *ctx, uint32_t *x, int32_t *found);
 /* n x n results of the last executed iteration (any may be NULL): vtAv, vtAAv,
  * winv are n*n, d is n; *npiv the value semi_inverse returned.            */
 int  blk_get_small(blk_ctx *ctx, uint32_t *vtAv, uint32_t *vtAAv, uint32_t *winv, uint32_t *d,
@@ -201,7 +214,7 @@ typedef struct blk_info {
         int64_t device_bytes;          /* resident bytes (matrix layouts + blocks) */
         int32_t loop_mode;             /* how blk_iterate runs the loop: 0 chain of kernels / CUDA graph, 1 one persistent
                                           cooperative kernel (L2-resident problems on one GPU, BLK_LOOP) */
-        int32_t reserved;
+        int32_t nrhs;                  /* right-hand sides of a blk_create_system context (counted in N), else 0 */
         int32_t bands[2];              /* column bands of S1 / S2 (0: none): n_pad <= 4 with an x block far larger than L2 */
 } blk_info;
 int  blk_get_info(blk_ctx *ctx, blk_info *info);
