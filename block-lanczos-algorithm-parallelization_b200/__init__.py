@@ -23,11 +23,13 @@ BLK_ABI_VERSION = 2
 BLK_MAX_N = 64
 BLK_NCCL_ID_BYTES = 128
 BLK_RANK_ALL = -1          # blk_params.rank: one context (one process) drives all `world` GPUs
+PRUNE_STATS = ("N", "Mc", "nnz", "free", "rounds")     # BLK_PR_N ... BLK_PR_ROUNDS
 PHASES = ("spmv1", "spmv2", "dots", "small", "ortho", "exchange")
 
 # every symbol include/blk_lanczos.h declares
 ABI_SYMBOLS = (
     "blk_abi_version", "blk_last_error", "blk_device_count", "blk_nccl_unique_id", "blk_create", "blk_create_system",
+    "blk_create_pruned", "blk_pruned_index",
     "blk_destroy", "blk_plan_shards", "blk_plan_grid", "blk_block_pad", "blk_set_state", "blk_iterate", "blk_get_state", "blk_get_state_local", "blk_final_check",
     "blk_check_kernel_block", "blk_kernel_basis", "blk_solve", "blk_get_small",
     "blk_spmv", "blk_block_dot_products", "blk_semi_inverse", "blk_orthogonalize",
@@ -79,6 +81,8 @@ def load_library(path: str | None = None) -> C.CDLL:
     L.blk_nccl_unique_id.argtypes = [vp]
     L.blk_create.argtypes = [C.POINTER(vp), C.POINTER(blk_params)]
     L.blk_create_system.argtypes = [C.POINTER(vp), C.POINTER(blk_params), vp, i32, i32]
+    L.blk_create_pruned.argtypes = [C.POINTER(vp), C.POINTER(blk_params), vp]
+    L.blk_pruned_index.argtypes = [vp, vp, vp]
     L.blk_destroy.argtypes = [vp]
     L.blk_plan_shards.argtypes = [vp, i64, i64, i32, vp]
     L.blk_plan_grid.argtypes = [vp, vp, i64, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp]
@@ -173,7 +177,8 @@ class BlockLanczos:
 
     def __init__(self, M=None, *, n: int, prime: int, right: bool = False, device: int = 0,
                  rank: int = 0, world: int = 1, nccl_id: bytes | None = None, stream: int | None = None,
-                 chunk_len: int = 0, use_graph: int = -1, device_coo=None, rhs=None, rhs_device=None):
+                 chunk_len: int = 0, use_graph: int = -1, device_coo=None, rhs=None, rhs_device=None,
+                 prune: bool = False):
         """`M` is a host SparseCOO; alternatively `device_coo=(nrows, ncols, nnz, i_ptr, j_ptr, x_ptr)`
         gives raw CUDA device pointers (int32, int32, uint32) on `device`.  `rank=BLK_RANK_ALL` with
         `world=W` makes ONE context drive W GPUs (devices device..device+W-1) from this process.
@@ -182,9 +187,16 @@ class BlockLanczos:
         the system M x = b (x M = b for --left), blk_create_system: the loop then runs on the augmented matrix, so
         `nrows` / `ncols` / `N` / `pad` are its sizes; `N0` is the original length and `nrhs` = r.  Negative
         entries are taken like the MatrixMarket loader takes them (-k is 2^32 - k before the reduction mod p).
-        `rhs_device=(ptr, r)` gives that block instead as a raw CUDA device pointer (uint32, Mc x r) on `device`."""
+        `rhs_device=(ptr, r)` gives that block instead as a raw CUDA device pointer (uint32, Mc x r) on `device`.
+
+        `prune=True` removes the empty and singleton constraints first (blk_create_pruned, DESIGN.md section 14): the
+        loop then runs on M', so `nrows` / `ncols` / `N` / `Mc` / `pad` are its sizes, `orig_N` / `orig_Mc` the
+        original ones; `prune_stats`, `pruned_index()` and `lift()` relate the two.  Not with `rhs`."""
         self.L = load_library()
         self.n, self.prime, self.right = int(n), int(prime), bool(right)
+        self.pruned, self.prune_stats = bool(prune), None
+        if prune and (rhs is not None or rhs_device is not None):
+            raise BlkError("prune=True cannot be combined with rhs= (a singleton constraint forces a value in a system)")
         prm = blk_params()
         prm.abi_version = BLK_ABI_VERSION
         keep = []
@@ -223,8 +235,11 @@ class BlockLanczos:
         prm.stream = stream
         prm.chunk_len, prm.use_graph = chunk_len, use_graph
         h = C.c_void_p()
+        stats = (C.c_int64 * len(PRUNE_STATS))()
         if self.nrhs:
             rc = self.L.blk_create_system(C.byref(h), C.byref(prm), b_ptr, self.nrhs, b_dev)
+        elif prune:
+            rc = self.L.blk_create_pruned(C.byref(h), C.byref(prm), stats)
         else:
             rc = self.L.blk_create(C.byref(h), C.byref(prm))
         del keep, idbuf
@@ -232,6 +247,13 @@ class BlockLanczos:
             raise BlkError(self.L.blk_last_error().decode())
         self.h = h
         self.N0 = self.ncols if right else self.nrows
+        self.orig_N, self.orig_Mc = self.N0, (self.nrows if right else self.ncols)
+        if prune:
+            self.prune_stats = {k: int(stats[i]) for i, k in enumerate(PRUNE_STATS)}
+            self.N0 = self.prune_stats["N"]
+            Mc = self.prune_stats["Mc"]
+            self.nrows, self.ncols = (Mc, self.N0) if right else (self.N0, Mc)
+            self.nnz = self.prune_stats["nnz"]
         if right:
             self.ncols += self.nrhs
         else:
@@ -355,6 +377,29 @@ class BlockLanczos:
         found = np.zeros(self.nrhs, dtype=np.int32)
         self._ck(self.L.blk_solve(self.h, _ptr(x), _ptr(found)))
         return x.reshape(self.N0, self.nrhs), found.astype(bool)
+
+    def pruned_index(self):
+        """(unknowns, constraints) of a context made with prune=True: the original indices of the N' kept unknowns and
+        the Mc' kept constraints, ascending int32 arrays (blk_pruned_index)."""
+        if not self.pruned:
+            raise BlkError("pruned_index() needs a context created with prune=True")
+        u = np.empty(self.N, dtype=np.int32)
+        c = np.empty(self.Mc, dtype=np.int32)
+        self._ck(self.L.blk_pruned_index(self.h, _ptr(u), _ptr(c)))
+        return u, c
+
+    def lift(self, x) -> np.ndarray:
+        """An N' x w block on the kept unknowns as the orig_N x w block of the original matrix, zero on the removed
+        unknowns (a kernel vector of M' lifts to a kernel vector of M)."""
+        x = np.asarray(x, dtype=np.uint32)
+        if x.ndim == 1:
+            x = x.reshape(self.N, -1)
+        if x.shape[0] != self.N:
+            raise BlkError(f"lift() takes an N' x w block (N' = {self.N}), got shape {x.shape}")
+        u, _ = self.pruned_index()
+        out = np.zeros((self.orig_N, x.shape[1]), dtype=np.uint32)
+        out[u] = x
+        return out
 
     def get_small(self):
         n = self.n

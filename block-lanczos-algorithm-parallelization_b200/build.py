@@ -18,7 +18,7 @@ DRIVER_DIR = os.path.join(PKG, "driver")
 DRIVER = os.path.join(DRIVER_DIR, "lanczos_modp")
 
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-CU_SOURCES = ["layout_build.cu", "spmv.cu", "dense.cu", "dense_mma.cu", "dense_umma.cu", "loop_coop.cu", "kernel_basis.cu", "solve.cu", "context.cu"]
+CU_SOURCES = ["layout_build.cu", "spmv.cu", "dense.cu", "dense_mma.cu", "dense_umma.cu", "loop_coop.cu", "kernel_basis.cu", "solve.cu", "prune.cu", "context.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "-ccbin", "/usr/bin/g++"]
 

@@ -325,3 +325,17 @@ int launch_solve_tail(const SolveArgs &a, int64_t N0, const u32 *v_full, const u
 int launch_solve_small(const SolveArgs &a, cudaStream_t st);
 // k_solve_apply: x = v W
 int launch_solve_apply(const SolveArgs &a, cudaStream_t st);
+// prune.cu: removal of empty and singleton constraints (blk_create_pruned), DESIGN.md section 14.
+struct PruneResult {
+        int64_t N = 0, Mc = 0, nnz = 0, free = 0, rounds = 0;    // kept unknowns, constraints, triplets; free unknowns; rounds
+        std::vector<int32_t> unknowns, constraints;              // original indices of the kept ones, ascending
+        bool identity = false;                                   // nothing removed: both maps are the identity (left empty)
+        int32_t *Mi = nullptr, *Mj = nullptr;                     // M' on the device (owned), or all null when M' is the input
+        u32 *Mx = nullptr;                                        // itself (nothing removed, no triplet vanishes mod p)
+        void release();
+        ~PruneResult() { release(); }
+};
+// The COO (device, values not reduced) of an nrows x ncols matrix, pruned as DESIGN.md section 14 defines it, on the
+// current device and stream st.  Returns an error message or "".
+std::string prune_coo(const int32_t *Mi, const int32_t *Mj, const u32 *Mx, int64_t nnz, int64_t nrows, int64_t ncols, int right,
+                      u32 p, cudaStream_t st, PruneResult *out);

@@ -102,6 +102,9 @@ struct blk_ctx {
         int32_t nrows = 0, ncols = 0;
         int64_t N = 0, Mc = 0;
         int nrhs = 0;                           // blk_create_system: right-hand sides appended to M (N counts them too)
+        bool pruned = false;                    // blk_create_pruned: original indices of the kept unknowns / constraints
+        bool pr_identity = false;               // (nothing removed: the identity, not stored)
+        std::vector<int32_t> pr_unknowns, pr_constraints;
         std::vector<int64_t> n_off, m_off;      // row partition of the N and Mc dimensions
         SpOp S1, S2;                            // tmp <- S1 v ; Av <- S2 tmp
         u32 *v = nullptr, *tmp = nullptr;       // full length: N*np, Mc*np
@@ -2151,8 +2154,99 @@ static int create_system(blk_ctx **out, const blk_params *prm, const uint32_t *B
 }
 
 
+// blk_create_pruned: the COO on prm->device (uploaded when it is on the host), pruned by prune_coo, handed to
+// blk_create as a device COO.  The upload is freed before blk_create, so that at most one extra copy of the COO
+// (M') is resident while the layouts are built.
+static int create_pruned(blk_ctx **out, const blk_params *prm, int64_t stats[BLK_PR_COUNT])
+{
+        if (!out) return fail("blk_create_pruned: null output pointer");
+        *out = nullptr;
+        if (!prm || prm->abi_version != BLK_ABI_VERSION) return fail("blk_params.abi_version mismatch");
+        if (prm->n < 1 || prm->n > BLK_MAX_N) return fail("blocking factor n must be in [1,64]");
+        if (prm->nrows < 1 || prm->ncols < 1 || prm->nnz < 0) return fail("bad matrix dimensions");
+        if (prm->nnz > 0 && (!prm->Mi || !prm->Mj || !prm->Mx)) return fail("null COO arrays");
+        ModP m;
+        if (!modp_make(&m, prm->prime)) return fail("prime must satisfy 2 <= p < 2^31");
+        const int right = prm->right_kernel ? 1 : 0;
+        int ndev = 0;
+        cudaError_t e0 = cudaGetDeviceCount(&ndev);
+        if (e0 != cudaSuccess || ndev == 0)
+                return fail(std::string("no CUDA device (there is no CPU fallback): ") + cudaGetErrorString(e0));
+        if (prm->device < 0 || prm->device >= ndev) return fail("device ordinal out of range");
+        CU(cudaSetDevice(prm->device));
+        struct Stream {
+                cudaStream_t st = nullptr;
+                ~Stream() { if (st) cudaStreamDestroy(st); }
+        } s;
+        CU(cudaStreamCreateWithFlags(&s.st, cudaStreamNonBlocking));
+        const int64_t nnz = prm->nnz;
+        Scratch up;
+        const int32_t *di = (const int32_t *)prm->Mi, *dj = (const int32_t *)prm->Mj;
+        const u32 *dx = (const u32 *)prm->Mx;
+        if (!prm->coo_on_device && nnz > 0) {
+                int32_t *hi = nullptr, *hj = nullptr;
+                u32 *hx = nullptr;
+                if (up.alloc(&hi, sizeof(int32_t) * (size_t)nnz) || up.alloc(&hj, sizeof(int32_t) * (size_t)nnz) ||
+                    up.alloc(&hx, sizeof(u32) * (size_t)nnz))
+                        return 1;
+                CU(cudaMemcpyAsync(hi, prm->Mi, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, s.st));
+                CU(cudaMemcpyAsync(hj, prm->Mj, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, s.st));
+                CU(cudaMemcpyAsync(hx, prm->Mx, sizeof(u32) * (size_t)nnz, cudaMemcpyHostToDevice, s.st));
+                di = hi; dj = hj; dx = hx;
+        }
+        PruneResult pr;
+        std::string err = prune_coo(di, dj, dx, nnz, prm->nrows, prm->ncols, right, m.p, s.st, &pr);
+        if (!err.empty()) return fail(err);
+        if (pr.Mc == 0) {
+                if (pr.N == 0) return fail("blk_create_pruned: pruning removed every unknown and every constraint: the kernel is {0}");
+                return fail("blk_create_pruned: pruning removed every constraint: every vector on the " + std::to_string(pr.N) +
+                            " surviving unknowns is a kernel vector");
+        }
+        if (stats) {
+                stats[BLK_PR_N] = pr.N; stats[BLK_PR_MC] = pr.Mc; stats[BLK_PR_NNZ] = pr.nnz;
+                stats[BLK_PR_FREE] = pr.free; stats[BLK_PR_ROUNDS] = pr.rounds;
+        }
+        blk_params p2 = *prm;
+        p2.nrows = (int32_t)(right ? pr.Mc : pr.N);
+        p2.ncols = (int32_t)(right ? pr.N : pr.Mc);
+        p2.nnz = pr.nnz; p2.coo_on_device = 1;
+        if (pr.Mx) {
+                for (void *q : up.ptrs) up.release(q);
+                p2.Mi = pr.Mi; p2.Mj = pr.Mj; p2.Mx = pr.Mx;
+        } else {
+                p2.Mi = di; p2.Mj = dj; p2.Mx = dx;
+        }
+        if (blk_create(out, &p2)) return 1;
+        blk_ctx *c = *out;
+        c->pruned = true;
+        c->pr_identity = pr.identity;
+        c->pr_unknowns = std::move(pr.unknowns);
+        c->pr_constraints = std::move(pr.constraints);
+        return 0;
+}
+
+
 // ---------------------------------------------------------------------------------- C ABI
 extern "C" {
+
+int blk_create_pruned(blk_ctx **out, const blk_params *prm, int64_t stats[BLK_PR_COUNT])
+{
+        return create_pruned(out, prm, stats);
+}
+
+int blk_pruned_index(blk_ctx *c, int32_t *unknowns, int32_t *constraints)
+{
+        if (!c) return fail("blk_pruned_index: null context");
+        if (!c->pruned) return fail("blk_pruned_index: the context was not made by blk_create_pruned");
+        if (c->pr_identity) {
+                if (unknowns) for (int64_t u = 0; u < c->N; u++) unknowns[u] = (int32_t)u;
+                if (constraints) for (int64_t m = 0; m < c->Mc; m++) constraints[m] = (int32_t)m;
+                return 0;
+        }
+        if (unknowns) std::copy(c->pr_unknowns.begin(), c->pr_unknowns.end(), unknowns);
+        if (constraints) std::copy(c->pr_constraints.begin(), c->pr_constraints.end(), constraints);
+        return 0;
+}
 
 int blk_abi_version(void) { return BLK_ABI_VERSION; }
 

@@ -13,6 +13,7 @@
  * USAGE:
  *      $ ./lanczos_modp --prime 65537 --n 4 --matrix random_small.mtx
  *      $ ./lanczos_modp --prime 65537 --n 16 --matrix M.mtx --rhs B.mtx --output-file X.mtx [--right]
+ *      $ ./lanczos_modp --prime 2 --n 64 --matrix M.mtx --prune --kernel-basis --output-file K.mtx
  *
  * Deviations from the reference, all documented in DESIGN.md:
  *   - p may be as large as 2^31-1 (the reference stops at 2^30-35);
@@ -27,6 +28,10 @@
  *     of the MatrixMarket array B (Mc x r, the format of the output file).  The loop runs on the augmented
  *     matrix [M | -B] (resp. [M ; -B^T]); blk_solve then extracts the solutions and the output file holds the
  *     N x r block X.  Exit status 1 and no file when some right-hand side is not solved;
+ *   - --prune (new): empty and singleton constraints are removed on the device before the loop
+ *     (blk_create_pruned); the loop, the final check and --kernel-basis run on the smaller matrix M', and the
+ *     output file is lifted back to the N rows of M (zeros on the removed unknowns).  Exit status 1 and no file
+ *     when every constraint is removed;
  *   - the GPU runs iterations in batches, so progress is reported per batch.
  */
 #define _POSIX_C_SOURCE 200809L
@@ -50,7 +55,7 @@ struct options {
         int n;
         bool right;
         int stop_after;
-        bool checkpoint, resume, kernel_basis;
+        bool checkpoint, resume, kernel_basis, prune;
         const char *rhs;
         double checkpoint_every;
         int device;
@@ -78,6 +83,7 @@ static void usage(const char *argv0)
         printf("--load-checkpoint           load vectors from checkpointing files\n");
         printf("--kernel-basis              store only independent kernel vectors (needs --output-file)\n");
         printf("--rhs FILENAME              solve M*X = B (X*M = B with --left) for the array B (needs --output-file)\n");
+        printf("--prune                     remove empty and singleton constraints before the loop\n");
         printf("\n");
         printf("The --matrix and --prime arguments are required\n");
         printf("The --stop-after and --output-file arguments mutually exclusive\n");
@@ -98,6 +104,7 @@ static void parse_options(struct options *o, int argc, char **argv)
                 {"load-checkpoint", no_argument, NULL, 'L'},
                 {"kernel-basis", no_argument, NULL, 'K'},
                 {"rhs", required_argument, NULL, 'B'},
+                {"prune", no_argument, NULL, 'P'},
                 {NULL, 0, NULL, 0}};
         memset(o, 0, sizeof(*o));
         o->n = 1;
@@ -126,6 +133,7 @@ static void parse_options(struct options *o, int argc, char **argv)
                 case 'L': o->resume = true; break;
                 case 'K': o->kernel_basis = true; break;
                 case 'B': o->rhs = optarg; break;
+                case 'P': o->prune = true; break;
                 default: errx(1, "Unknown option\n");
                 }
         }
@@ -137,6 +145,8 @@ static void parse_options(struct options *o, int argc, char **argv)
                 if (o->kernel_basis || o->stop_after > 0 || o->checkpoint || o->resume)
                         errx(1, "usage: --rhs cannot be combined with --kernel-basis, --stop-after, --checkpoint or --load-checkpoint");
         }
+        if (o->prune && (o->rhs || o->checkpoint || o->resume))
+                errx(1, "usage: --prune cannot be combined with --rhs, --checkpoint or --load-checkpoint");
         if (o->output && o->stop_after > 0)
                 usage(argv[0]);
         if (o->kernel_basis && !o->output)
@@ -340,6 +350,23 @@ static int gpus_from_env(void)
         return g;
 }
 
+/* The N x w block x (stride w) as the file of the original matrix: without --prune (kept == NULL) as it is, else
+ * lifted to its N_orig rows, zeros on the removed unknowns */
+static void save_lifted(const char *path, long N, long N_orig, int w, const uint32_t *x, const int32_t *kept)
+{
+        if (!kept) {
+                kernel_block_save(path, (int)N, w, x);
+                return;
+        }
+        uint32_t *big = calloc((size_t)N_orig * (size_t)w, sizeof(*big));
+        if (!big)
+                errx(1, "cannot allocate the lifted block");
+        for (long r = 0; r < N; r++)
+                memcpy(big + (size_t)kept[r] * w, x + (size_t)r * w, sizeof(*big) * (size_t)w);
+        kernel_block_save(path, (int)N_orig, w, big);
+        free(big);
+}
+
 int main(int argc, char **argv)
 {
         struct options o;
@@ -361,23 +388,8 @@ int main(int argc, char **argv)
                 if (nrhs > n)
                         errx(1, "%s has %d right-hand sides, more than the blocking factor n = %d", o.rhs, nrhs, n);
         }
-        const int anrows = M.nrows + (o.right ? 0 : nrhs), ancols = M.ncols + (o.right ? nrhs : 0);
-        const long N = o.right ? ancols : anrows;            /* length of the Lanczos vectors */
-        const long Mc = o.right ? anrows : ancols;
-        const long N0 = N - nrhs;                            /* the unknowns of the system */
-        const long pad = (long)blk_block_pad(anrows, ancols, n, o.right);
-
-        printf("Block Lanczos\n");
-        char hs[16];
-        human(hs, sizeof(hs), 4.0 * sizeof(int) * pad);
-        printf("  - Extra storage needed: %sB\n", hs);
-
-        uint32_t *v = calloc((size_t)pad, sizeof(*v));
-        uint32_t *tmp = calloc((size_t)pad, sizeof(*tmp));
-        uint32_t *Av = calloc((size_t)pad, sizeof(*Av));
-        uint32_t *p = calloc((size_t)pad, sizeof(*p));
-        if (!v || !tmp || !Av || !p)
-                errx(1, "impossible d'allouer les blocs de vecteur");
+        int anrows = M.nrows + (o.right ? 0 : nrhs), ancols = M.ncols + (o.right ? nrhs : 0);
+        const long orig_N = o.right ? M.ncols : M.nrows, orig_Mc = o.right ? M.nrows : M.ncols, orig_nnz = M.nnz;
 
         blk_params prm;
         memset(&prm, 0, sizeof(prm));
@@ -390,9 +402,43 @@ int main(int argc, char **argv)
         prm.world = gpus; prm.rank = gpus > 1 ? BLK_RANK_ALL : 0;
         blk_ctx *ctx = NULL;
         double t_build = wall();
+        /* --prune: the context of M' comes first, its sizes are those of the loop */
+        int64_t pst[BLK_PR_COUNT] = {0};
+        int32_t *kept = NULL;                                /* original indices of the kept unknowns */
+        printf("Block Lanczos\n");
+        if (o.prune) {
+                GPU(blk_create_pruned(&ctx, &prm, pst));
+                printf("  - Prune: kept %" PRId64 " of %ld unknowns (%" PRId64 " free), %" PRId64 " of %ld constraints, "
+                       "%" PRId64 " of %ld entries in %" PRId64 " rounds, %.2f s\n", pst[BLK_PR_N], orig_N, pst[BLK_PR_FREE],
+                       pst[BLK_PR_MC], orig_Mc, pst[BLK_PR_NNZ], orig_nnz, pst[BLK_PR_ROUNDS], wall() - t_build);
+                anrows = (int)(o.right ? pst[BLK_PR_MC] : pst[BLK_PR_N]);
+                ancols = (int)(o.right ? pst[BLK_PR_N] : pst[BLK_PR_MC]);
+                kept = malloc(sizeof(*kept) * (size_t)pst[BLK_PR_N]);
+                if (!kept)
+                        errx(1, "cannot allocate the index map");
+                GPU(blk_pruned_index(ctx, kept, NULL));
+        }
+        const long N = o.right ? ancols : anrows;            /* length of the Lanczos vectors */
+        const long Mc = o.right ? anrows : ancols;
+        const long N0 = N - nrhs;                            /* the unknowns of the system */
+        const long pad = (long)blk_block_pad(anrows, ancols, n, o.right);
+
+        char hs[16];
+        human(hs, sizeof(hs), 4.0 * sizeof(int) * pad);
+        printf("  - Extra storage needed: %sB\n", hs);
+
+        uint32_t *v = calloc((size_t)pad, sizeof(*v));
+        uint32_t *tmp = calloc((size_t)pad, sizeof(*tmp));
+        uint32_t *Av = calloc((size_t)pad, sizeof(*Av));
+        uint32_t *p = calloc((size_t)pad, sizeof(*p));
+        if (!v || !tmp || !Av || !p)
+                errx(1, "impossible d'allouer les blocs de vecteur");
+
+        if (!o.prune)
+                t_build = wall();
         if (o.rhs)
                 GPU(blk_create_system(&ctx, &prm, B, nrhs, 0));
-        else
+        else if (!o.prune)
                 GPU(blk_create(&ctx, &prm));
         free(B);
         if (gpus > 1)
@@ -515,12 +561,12 @@ int main(int argc, char **argv)
                 for (long r = 0; r < N; r++)                 /* N x n, stride n -> N x k, stride k */
                         for (int j = 0; j < k; j++)
                                 Av[r * k + j] = tmp[r * n + j];
-                kernel_block_save(o.output, (int)N, (int)k, Av);
+                save_lifted(o.output, N, orig_N, (int)k, Av, kept);
         } else if (o.output)
-                kernel_block_save(o.output, (int)N, n, v);
+                save_lifted(o.output, N, orig_N, n, v, kept);
         else
                 printf("Not saving result (no --output given)\n");
         blk_destroy(ctx);
-        free(v); free(tmp); free(Av); free(p);
+        free(v); free(tmp); free(Av); free(p); free(kept);
         return EXIT_SUCCESS;
 }

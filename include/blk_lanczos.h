@@ -87,6 +87,19 @@ int  blk_create(blk_ctx **out, const blk_params *prm);
  * every other entry point works on it, the Lanczos vectors have N + nrhs rows (blk_block_pad, blk_get_info().N),
  * the last nrhs of them the coordinates of the right-hand sides.  rank / world / BLK_RANK_ALL as for blk_create. */
 int  blk_create_system(blk_ctx **out, const blk_params *prm, const uint32_t *B, int32_t nrhs, int32_t b_on_device);
+/* Removal of empty and singleton constraints before the loop (DESIGN.md section 14).  Unknowns are the coordinates of
+ * the Lanczos vectors (rows of M for --left, columns for --right), constraints the other dimension.  Rounds remove
+ * every constraint with at most one counting triplet (x mod p != 0) on a kept unknown, and that unknown, until none
+ * is left; the kernel is unchanged up to zeros on the removed unknowns.  The context is blk_create's for M', the kept
+ * counting triplets renumbered by rank (every other entry point works on M': blk_get_info().N / Mc, blk_block_pad,
+ * the state blocks, ...).  Same inputs as blk_create (host or device COO, rank / world / BLK_RANK_ALL; with one
+ * process per rank every rank prunes the whole COO itself).  Fails when every constraint is removed. */
+enum { BLK_PR_N = 0, BLK_PR_MC = 1, BLK_PR_NNZ = 2, BLK_PR_FREE = 3, BLK_PR_ROUNDS = 4, BLK_PR_COUNT = 5 };
+/* blk_create on M' (see DESIGN.md section 14); stats (nullable) receives N', Mc', nnz', free unknowns, rounds. */
+int  blk_create_pruned(blk_ctx **out, const blk_params *prm, int64_t stats[BLK_PR_COUNT]);
+/* Original indices of the kept unknowns [N'] and constraints [Mc'], ascending (either may be NULL);
+ * fails on a context not made by blk_create_pruned. */
+int  blk_pruned_index(blk_ctx *ctx, int32_t *unknowns, int32_t *constraints);
 int  blk_destroy(blk_ctx *ctx);
 
 /* Host-only: the contiguous, weight-balanced row partition blk_create uses for a `world`-GPU job.
