@@ -30,7 +30,7 @@ PHASES = ("spmv1", "spmv2", "dots", "small", "ortho", "exchange")
 ABI_SYMBOLS = (
     "blk_abi_version", "blk_last_error", "blk_device_count", "blk_nccl_unique_id", "blk_create", "blk_create_system",
     "blk_create_pruned", "blk_pruned_index",
-    "blk_destroy", "blk_plan_shards", "blk_plan_grid", "blk_block_pad", "blk_set_state", "blk_iterate", "blk_get_state", "blk_get_state_local", "blk_final_check",
+    "blk_destroy", "blk_plan_shards", "blk_plan_grid", "blk_plan_heavy", "blk_block_pad", "blk_set_state", "blk_iterate", "blk_get_state", "blk_get_state_local", "blk_final_check",
     "blk_check_kernel_block", "blk_kernel_basis", "blk_solve", "blk_get_small",
     "blk_spmv", "blk_block_dot_products", "blk_semi_inverse", "blk_orthogonalize",
     "blk_set_profiling", "blk_get_phase_times", "blk_time_spmv", "blk_kernel_launches", "blk_get_info",
@@ -58,6 +58,7 @@ class blk_info(C.Structure):
         ("stored_local", C.c_int64 * 2), ("tiles", C.c_int64 * 2), ("n", C.c_int32), ("n_pad", C.c_int32),
         ("chunk_len", C.c_int32 * 2), ("groups_per_warp", C.c_int32), ("device_bytes", C.c_int64),
         ("loop_mode", C.c_int32), ("nrhs", C.c_int32), ("bands", C.c_int32 * 2),
+        ("heavy_rows", C.c_int64), ("heavy_bands", C.c_int32),
     ]
 
 
@@ -86,6 +87,7 @@ def load_library(path: str | None = None) -> C.CDLL:
     L.blk_destroy.argtypes = [vp]
     L.blk_plan_shards.argtypes = [vp, i64, i64, i32, vp]
     L.blk_plan_grid.argtypes = [vp, vp, i64, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp]
+    L.blk_plan_heavy.argtypes = [vp, i64, i64, i32, i64, i64, i64, i32, C.POINTER(i64), C.POINTER(i32)]
     L.blk_block_pad.argtypes = [i32, i32, i32, i32]
     L.blk_block_pad.restype = i64
     L.blk_set_state.argtypes = [vp, vp, vp, i32]
@@ -134,6 +136,16 @@ def plan_shards(idx, dim: int, world: int) -> np.ndarray:
     if L.blk_plan_shards(_ptr(idx), idx.size, dim, world, _ptr(off)):
         raise BlkError(L.blk_last_error().decode())
     return off
+
+
+def plan_heavy(deg, cols: int, n_pad: int, l2_bytes: int, min_deg: int, band_bytes: int, force: bool = False):
+    """(H, K) of blk_plan_heavy (host only): the high-degree row prefix of product 2 run as K column bands."""
+    L = load_library()
+    deg = _u32(deg)
+    H, K = C.c_int64(0), C.c_int32(0)
+    if L.blk_plan_heavy(_ptr(deg), deg.size, cols, n_pad, l2_bytes, min_deg, band_bytes, int(force), C.byref(H), C.byref(K)):
+        raise BlkError(L.blk_last_error().decode())
+    return H.value, K.value
 
 
 def plan_grid(M, right: bool, world: int, grid=(0, 0)) -> dict:

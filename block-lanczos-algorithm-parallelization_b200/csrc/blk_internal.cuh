@@ -64,7 +64,27 @@ struct SpOp {
         u32 *rowmap = nullptr;     // this operator is a compact band: output row r -> y row rowmap[r], results accumulate
         u32 hot_cols = 0;          // > 0: entries carry a HOT bit (bit 30 of the column word): those x rows are gathered with
                                    // L2 evict_last, the rest evict_first (columns are then limited to 2^30)
+        // Heavy/light split (product 2, n_pad >= 8, one GPU, degree-sorted rows): the operator is ALSO stored as two operators.
+        // split[0] holds the high-degree row prefix [0, H) cut into heavy_bands = K column bands as ONE stream over K * H
+        // virtual rows, row b * H + r = (band b, row r): its output rows are the K band-major partial blocks in zheavy
+        // (H * n_pad words each), its tiles run band after band in one launch, and k_band_combine adds the partials into
+        // y[0, H).  split[1] is an ordinary operator over rows [H, rows) whose output starts at row H.  A partial costs
+        // n_pad words per heavy row and band, while the band's L2-resident x slice saves a line per non-zero.  launch_spmv
+        // dispatches here for unpieced, unpushed calls; everything else keeps using the full operator.
+        std::vector<SpOp> split;
+        int64_t heavy_rows = 0;
+        int heavy_bands = 0;
+        u32 *zheavy = nullptr;
 };
+
+// The heavy prefix of product 2 (SpOp::split): rows whose degree is >= min_deg, run as column bands of band_bytes of x each.
+// deg: row degrees under the degree-sorted labels (non-increasing).  force: skip the size and cost checks (tests).
+struct HeavyPlan {
+        int64_t rows = 0;          // H (0: no split)
+        int bands = 0;             // K
+};
+HeavyPlan plan_heavy(const u32 *deg, int64_t rows, int64_t cols, int np, int64_t l2_bytes, int64_t min_deg, int64_t band_bytes,
+                     bool force);
 
 // n x n working set of one iteration, resident on the device.  All matrices are stored with
 // leading dimension n_pad (zero padded) so the row kernels can use them directly.

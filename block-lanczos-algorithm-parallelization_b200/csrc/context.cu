@@ -1383,16 +1383,43 @@ int kernels_per_iteration(const blk_ctx *c)
 {
         // two products (+ their k_spmv_fix unless the rows crossing tiles are finished by look-back; banded products: every band
         // plus the pass that adds the partial results), dots, [small], orthogonalize
-        auto product = [](const SpOp &op) {
+        auto banded = [](const SpOp &op) {
                 if (op.bands.empty()) return op.lookback ? 1 : 2;
                 int k = 1;
                 for (const SpOp &b : op.bands) k += b.lookback ? 1 : 2;
                 return k;
         };
+        auto product = [&](const SpOp &op) {
+                if (op.split.empty()) return banded(op);
+                return banded(op.split[0]) + 1 + (op.split[1].rows > 0 ? banded(op.split[1]) : 0);
+        };
         return product(c->S1) + product(c->S2) + 1 + (c->fuse_small ? 0 : 1) + 1;
 }
 
 }  // namespace
+
+HeavyPlan plan_heavy(const u32 *deg, int64_t rows, int64_t cols, int np, int64_t l2_bytes, int64_t min_deg, int64_t band_bytes,
+                     bool force)
+{
+        HeavyPlan plan;
+        const int64_t x_bytes = cols * np * 4;
+        if (np < 8 || rows <= 0 || cols <= 0 || band_bytes <= 0 || (!force && x_bytes <= l2_bytes)) return plan;
+        const int64_t K = std::min<int64_t>(256, (x_bytes + band_bytes - 1) / band_bytes);
+        if (K < 2) return plan;
+        int64_t H = 0, heavy_nnz = 0;
+        while (H < rows && (int64_t)deg[H] >= min_deg) heavy_nnz += deg[H++];
+        if (H == 0) return plan;
+        // Bytes of HBM time per iteration: every heavy non-zero stops fetching its own line from HBM but still gathers from its
+        // band's slice (measured on config 4: 71 G gathers/s against ~5.9 TB/s, worth ~83 bytes); every (heavy row, band)
+        // writes and reads a partial row of 4 * n_pad bytes and streams one dummy entry when the row has nothing in the band.
+        // (At n_pad = 32 this says no, and the split measured slower there: 40.3 against 37.7 ms per product.)
+        const double line = std::max(128, 4 * np), l2_gather = 83.0;
+        const double saving = (line - l2_gather) * (double)heavy_nnz - (8.0 * np + 8.0) * (double)H * (double)K;
+        if (!force && saving <= 0) return plan;
+        plan.rows = H;
+        plan.bands = (int)K;
+        return plan;
+}
 
 // ---- blk_create, in pieces ------------------------------------------------------------------------
 namespace {
@@ -1625,6 +1652,91 @@ int build_bands(blk_ctx *c, SpOp *op, int K, int chunk_len, int64_t count, const
         CU(cudaMalloc(&op->zband, zb));
         CU(cudaMemsetAsync(op->zband, 0, zb, c->stream));
         op->bytes += zb;
+        return 0;
+}
+
+// row r of an entry in column c -> virtual row b * H + r of the band-major heavy operator, b = the band holding c
+// (band b covers the columns [cols * b / K, cols * (b + 1) / K))
+__global__ void k_band_rows(int64_t count, int32_t *__restrict__ row, const int32_t *__restrict__ col, int64_t cols, int K, int64_t H)
+{
+        int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+        if (s >= count) return;
+        const int64_t c = col[s];
+        int64_t b = c * K / cols;
+        while (b + 1 < K && cols * (b + 1) / K <= c) b++;
+        while (b > 0 && cols * b / K > c) b--;
+        row[s] = (int32_t)(b * H + row[s]);
+}
+
+// Heavy/light split of product 2 (SpOp::split, plan_heavy): S2's rows are the degree-sorted N dimension, so its H heaviest
+// rows are the label prefix [0, H).  The entries (rkey, ckey, val)[nnz] carry the ORIGINAL labels; n_old2new relabels the
+// rows.  Like bands, the split is an optimisation: skipped (return 0, no split) when the device cannot hold it.
+int build_heavy_split(blk_ctx *c, SpOp *op, int chunk_len, int64_t nnz, const int32_t *rkey, const int32_t *ckey, const u32 *val)
+{
+        const int np = c->geo.np;
+        const char *e = getenv("BLK_HEAVY"), *ed = getenv("BLK_HEAVY_MIN_DEG"), *eb = getenv("BLK_HEAVY_BAND_BYTES");
+        if ((e && e[0] == '0') || !c->n_old2new || c->world != 1 || np < 8 || nnz <= 0) return 0;
+        // defaults: the fastest point of the sweep on the config-4 matrix (DESIGN.md section 4, profiles/r05_heavy_bands.json)
+        const int64_t min_deg = ed ? atoll(ed) : 200;
+        const int64_t band_bytes = eb ? std::max(4096ll, atoll(eb)) : 48ll << 20;
+        int l2 = 0;
+        if (cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, c->device) != cudaSuccess) { cudaGetLastError(); return 0; }
+        std::vector<u32> deg;
+        if (count_dimension(c, nnz, rkey, c->N, &deg, c->n_old2new)) return 1;
+        const HeavyPlan plan = plan_heavy(deg.data(), c->N, c->Mc, np, l2, min_deg, band_bytes, env_flag("BLK_HEAVY_FORCE"));
+        if (plan.rows == 0) return 0;
+        const int64_t H = plan.rows, K = plan.bands;
+        if (H * K >= (1ll << 31)) return 0;
+        int64_t cnt_part[2] = {0, 0};
+        for (int64_t r = 0; r < c->N; r++) cnt_part[r < H ? 0 : 1] += deg[(size_t)r];
+        std::vector<u32>().swap(deg);
+
+        op->split.assign(2, SpOp());
+        SpOp &heavy = op->split[0], &light = op->split[1];
+        auto give_up = [&]() {
+                for (auto &s : op->split) free_operator(&s);
+                op->split.clear();
+                cudaFree(op->zheavy); op->zheavy = nullptr;
+                return 0;
+        };
+        Scratch tmp;
+        unsigned long long *cnt = nullptr;
+        if (tmp.alloc(&cnt, sizeof(unsigned long long))) return 1;
+        for (int part = 0; part < 2; part++) {
+                const int64_t lo = part ? H : 0, hi = part ? c->N : H, sel = cnt_part[part];
+                const int64_t rows = part ? hi - lo : K * H;
+                {
+                        // selection (12 B), the builder's sort (24 B) and the stream (8 B) per entry, one dummy entry and the
+                        // builder's row arrays per (virtual) row, the partial blocks
+                        size_t free_b = 0, total_b = 0;
+                        const double need = 44.0 * sel + 32.0 * rows + (part ? 0.0 : 4.0 * np * rows);
+                        if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess || need > 0.85 * (double)free_b) {
+                                cudaGetLastError();
+                                return give_up();
+                        }
+                }
+                Scratch buf;
+                int32_t *sr = nullptr, *sc = nullptr; u32 *sx = nullptr;
+                unsigned long long h = 0;
+                if (buf.alloc(&sr, sizeof(int32_t) * (size_t)sel) || buf.alloc(&sc, sizeof(int32_t) * (size_t)sel) ||
+                    buf.alloc(&sx, sizeof(u32) * (size_t)sel))
+                        return 1;
+                CU(cudaMemsetAsync(cnt, 0, sizeof(unsigned long long), c->stream));
+                k_select_range<<<nb(nnz), 256, 0, c->stream>>>(nnz, rkey, ckey, val, lo, hi, sr, sc, sx, cnt, c->n_old2new, c->N, nullptr, c->Mc);
+                CU(cudaMemcpyAsync(&h, cnt, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
+                CU(cudaStreamSynchronize(c->stream));
+                if ((int64_t)h != sel) return fail("heavy split selection count mismatch");
+                if (part == 0 && sel) k_band_rows<<<nb(sel), 256, 0, c->stream>>>(sel, sr, sc, c->Mc, (int)K, H);
+                std::string err = build_operator(part ? &light : &heavy, c->geo, chunk_len, rows, c->Mc, lo, sel, sr, sc, sx, c->m.p,
+                                                 nullptr, nullptr, 1, c->stream, nullptr);
+                if (!err.empty()) return fail(std::string("heavy split, ") + (part ? "light rows: " : "heavy rows: ") + err);
+        }
+        const size_t zb = sizeof(u32) * (size_t)(K * H) * np;
+        CU(cudaMalloc(&op->zheavy, zb));
+        CU(cudaMemsetAsync(op->zheavy, 0, zb, c->stream));
+        op->heavy_rows = H;
+        op->heavy_bands = (int)K;
+        op->bytes += heavy.bytes + light.bytes + zb;
         return 0;
 }
 
@@ -1885,6 +1997,7 @@ int create_impl(blk_ctx *c, const blk_params *prm)
                             build_colops(c, which ? &c->cb2 : &c->cb1, c->colblocks, prm->chunk_len, nnz, rk, ck, dx, lo, hi, cols,
                                          which ? c->m_off : c->n_off))
                                 return 1;
+                        if (err.empty() && which && !c->colblocks && build_heavy_split(c, op, prm->chunk_len, nnz, rk, ck, dx)) return 1;
                 } else {
                         Scratch sel_buf;
                         int32_t *sr = nullptr, *sc = nullptr; u32 *sx = nullptr;
@@ -1961,7 +2074,7 @@ int create_impl(blk_ctx *c, const blk_params *prm)
                 if (e && !force && !off && strcmp(e, "auto")) return fail("BLK_LOOP must be graph, coop or auto");
                 const size_t working_set = c->S1.bytes + c->S2.bytes + c->block_bytes - 2 * blk_ctx::STAGE_BYTES;
                 const bool eligible = world == 1 && !c->colblocks && loop_coop_supported(np) && !c->S1.lookback && !c->S2.lookback &&
-                                      !c->S1.hot_cols && c->S1.bands.empty() && c->S2.bands.empty() && c->N > 0 && c->Mc > 0;
+                                      !c->S1.hot_cols && c->S1.bands.empty() && c->S2.bands.empty() && c->S2.split.empty() && c->N > 0 && c->Mc > 0;
                 if (force && !eligible) return fail("BLK_LOOP=coop: the persistent loop kernel needs one GPU, n <= 16 and the default product kernels");
                 (void)working_set;
                 if (eligible && force) {
@@ -2287,6 +2400,16 @@ int blk_plan_shards(const int32_t *idx, int64_t nnz, int64_t dim, int32_t world,
         }
         std::vector<int64_t> off = partition_rows(cnt, world);
         for (int r = 0; r <= world; r++) offsets[r] = off[r];
+        return 0;
+}
+
+int blk_plan_heavy(const uint32_t *deg, int64_t rows, int64_t cols, int32_t n_pad, int64_t l2_bytes, int64_t min_deg,
+                   int64_t band_bytes, int32_t force, int64_t *heavy_rows, int32_t *bands)
+{
+        if (!heavy_rows || !bands || rows < 0 || cols < 0 || (rows > 0 && !deg)) return fail("blk_plan_heavy: bad argument");
+        const HeavyPlan plan = plan_heavy(deg, rows, cols, n_pad, l2_bytes, min_deg, band_bytes, force != 0);
+        *heavy_rows = plan.rows;
+        *bands = plan.bands;
         return 0;
 }
 
@@ -3154,6 +3277,7 @@ int blk_get_info(blk_ctx *c, blk_info *info)
         info->device_bytes = (int64_t)(c->S1.bytes + c->S2.bytes + c->block_bytes);
         info->loop_mode = (c->coop && c->use_graph != 0) ? 1 : 0;
         info->bands[0] = (int32_t)c->S1.bands.size(); info->bands[1] = (int32_t)c->S2.bands.size();
+        info->heavy_rows = c->S2.heavy_rows; info->heavy_bands = c->S2.heavy_bands;
         return 0;
 }
 

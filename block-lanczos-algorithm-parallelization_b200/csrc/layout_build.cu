@@ -144,7 +144,8 @@ void free_operator(SpOp *op)
         cudaFree(op->ent); cudaFree(op->chunk_row); cudaFree(op->tail_row);
         cudaFree(op->span); cudaFree(op->whead); cudaFree(op->back); cudaFree(op->ready);
         for (auto &b : op->bands) free_operator(&b);
-        cudaFree(op->zband); cudaFree(op->rowmap);
+        for (auto &s : op->split) free_operator(&s);
+        cudaFree(op->zband); cudaFree(op->rowmap); cudaFree(op->zheavy);
         *op = SpOp();
 }
 

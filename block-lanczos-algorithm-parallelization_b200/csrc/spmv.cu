@@ -165,11 +165,40 @@ k_band_combine1(u32 *__restrict__ y, const u32 *__restrict__ z, int K, size_t st
         }
 }
 
+// y[0, stride) <- sum of the K partial blocks z + b * stride, mod p
+int launch_combine(u32 *y, const u32 *z, int K, size_t stride, const ModP &m, const DevSmall *state, cudaStream_t st)
+{
+        int k = 0;
+        const int64_t count = (int64_t)stride;
+        const bool vec = (stride % 4) == 0 && ((uintptr_t)y % 16) == 0;
+        const int64_t count4 = vec ? count / 4 : 0;
+        if (count4 > 0) {
+                unsigned blocks = (unsigned)std::min<int64_t>((int64_t)blk_sm_count() * 16, (count4 + 255) / 256);
+                launch_k(k_band_combine, blocks, 256, 0, st, y, z, K, stride, count4, m, state);
+                k++;
+        }
+        if (count4 * 4 < count) {
+                unsigned blocks = (unsigned)std::min<int64_t>((int64_t)blk_sm_count() * 16, (count - count4 * 4 + 255) / 256);
+                launch_k(k_band_combine1, blocks, 256, 0, st, y, z, K, stride, count4 * 4, count, m, state);
+                k++;
+        }
+        return k;
+}
+
 }  // namespace
 
 int launch_spmv(const SpOp &op, const Geometry &geo, const ModP &m, const u32 *x, u32 *y,
                 const DevSmall *state, cudaStream_t st, int piece, const PushTargets *push)
 {
+        if (!op.split.empty() && (piece < 0 || op.piece_tile.size() <= 2) && !(push && push->n > 0)) {
+                // heavy prefix as column bands (one launch, band after band, into the partial blocks; then the pass that adds
+                // them into y[0, H)), then the light rows -- one after the other, so that the light product's random gathers
+                // do not evict the bands' x slices
+                const size_t stride = (size_t)op.heavy_rows * geo.np;
+                int k = launch_spmv(op.split[0], geo, m, x, op.zheavy, state, st);
+                k += launch_combine(y, op.zheavy, op.heavy_bands, stride, m, state, st);
+                return k + launch_spmv(op.split[1], geo, m, x, y + stride, state, st);
+        }
         if (!op.bands.empty() && (piece < 0 || op.piece_tile.size() <= 2) && !(push && push->n > 0)) {
                 // column bands: K products whose x slices are L2-resident, then one pass that adds the partial results
                 const int K = (int)op.bands.size();
@@ -183,20 +212,7 @@ int launch_spmv(const SpOp &op, const Geometry &geo, const ModP &m, const u32 *x
                         return k;
                 }
                 for (int b = 0; b < K; b++) k += launch_spmv(op.bands[b], geo, m, x, op.zband + (size_t)b * stride, state, st);
-                const int64_t count = (int64_t)stride;
-                const bool vec = (stride % 4) == 0 && ((uintptr_t)y % 16) == 0;
-                const int64_t count4 = vec ? count / 4 : 0;
-                if (count4 > 0) {
-                        unsigned blocks = (unsigned)std::min<int64_t>((int64_t)blk_sm_count() * 16, (count4 + 255) / 256);
-                        launch_k(k_band_combine, blocks, 256, 0, st, y, (const u32 *)op.zband, K, stride, count4, m, state);
-                        k++;
-                }
-                if (count4 * 4 < count) {
-                        unsigned blocks = (unsigned)std::min<int64_t>((int64_t)blk_sm_count() * 16, (count - count4 * 4 + 255) / 256);
-                        launch_k(k_band_combine1, blocks, 256, 0, st, y, (const u32 *)op.zband, K, stride, count4 * 4, count, m, state);
-                        k++;
-                }
-                return k;
+                return k + launch_combine(y, op.zband, K, stride, m, state, st);
         }
         switch (geo.np) {
         case 1: return launch_lv<1, 1>(op, m, x, y, state, st, piece, push);

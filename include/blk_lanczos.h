@@ -127,6 +127,15 @@ int  blk_plan_grid(const int32_t *Mi, const int32_t *Mj, int64_t nnz, int32_t nr
                    int32_t right_kernel, int32_t world, int32_t grid[2], int64_t *n_off, int64_t *m_off,
                    int64_t *n_sub, int64_t *m_sub, int64_t *block_nnz);
 
+/* Host-only: the heavy prefix of product 2 that blk_create runs as column bands on one GPU (DESIGN.md section 4).
+ * deg[rows] are the row degrees of that product under the degree-sorted labels (non-increasing), cols the length
+ * of the block it gathers, l2_bytes the device's L2.  *heavy_rows receives H, the rows with degree >= min_deg, and
+ * *bands K = ceil(cols * n_pad * 4 / band_bytes) (<= 256); both 0 when no split pays: n_pad < 8, a gathered block
+ * that fits L2, or a predicted saving (lines not fetched minus partial traffic and the bands' gather time) <= 0.
+ * force skips the last two checks. */
+int  blk_plan_heavy(const uint32_t *deg, int64_t rows, int64_t cols, int32_t n_pad, int64_t l2_bytes, int64_t min_deg,
+                    int64_t band_bytes, int32_t force, int64_t *heavy_rows, int32_t *bands);
+
 /* block_size_pad of block_lanczos (:594-597) in u32 elements: the length of the
  * reference's v/tmp/Av/p blocks and of every block in blk_get_state. */
 int64_t blk_block_pad(int32_t nrows, int32_t ncols, int32_t n, int32_t right_kernel);
@@ -229,6 +238,8 @@ typedef struct blk_info {
                                           cooperative kernel (L2-resident problems on one GPU, BLK_LOOP) */
         int32_t nrhs;                  /* right-hand sides of a blk_create_system context (counted in N), else 0 */
         int32_t bands[2];              /* column bands of S1 / S2 (0: none): n_pad <= 4 with an x block far larger than L2 */
+        int64_t heavy_rows;            /* rows of S2's heavy prefix run as column bands (0: no split, blk_plan_heavy) */
+        int32_t heavy_bands;           /* its column bands */
 } blk_info;
 int  blk_get_info(blk_ctx *ctx, blk_info *info);
 
