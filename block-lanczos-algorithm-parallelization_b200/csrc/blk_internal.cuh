@@ -311,15 +311,14 @@ struct KbArgs {
         u32 *rec_all = nullptr;        // [world][2] records
         u32 *A = nullptr;              // n_pad x n_pad: A_S, column s = a_f of the s-th vector
         int *k = nullptr;              // number of kernel vectors
-        u32 *x = nullptr;              // vrows x n_pad: X = v A_S
 };
 int kb_ctas(int64_t rows);
 // k_kb_reduce: both blocks -> rec_own
 int launch_kb_reduce(int np, const KbArgs &a, cudaStream_t st);
 // k_kb_small: rec_all -> A, k
 int launch_kb_small(int np, const KbArgs &a, cudaStream_t st);
-// k_kb_apply: x = v A
-int launch_kb_apply(int np, const KbArgs &a, cudaStream_t st);
+// k_block_apply: x = v W for `rows` rows of v (n_pad words each), W n_pad x wp (wp a power of two <= n_pad), x wp words a row
+int launch_block_apply(int np, int wp, int64_t rows, const u32 *v, const u32 *W, u32 *x, const ModP &m, cudaStream_t st);
 // solve.cu: inhomogeneous systems (blk_create_system, blk_solve), DESIGN.md section 13.
 // The non-zeros of -B (Mc x r, row-major, device) as COO triplets of the augmented matrix: (i, N + j) for --right,
 // (N + j, i) for --left.  *count receives their number; with Mi == nullptr nothing is written (a first call sizes the
@@ -335,16 +334,11 @@ struct SolveArgs {
         u32 *tail = nullptr;           // r x n_pad: the tail rows of v (rows N .. N+r-1 of the augmented problem)
         u32 *W = nullptr;              // n_pad x rp: W = A_S C
         int *found = nullptr;          // [r]
-        const u32 *v = nullptr;        // this rank's rows of v (vrows x n_pad)
-        int64_t vrows = 0;
-        u32 *x = nullptr;              // vrows x rp: x = v W
 };
 // k_solve_tail: the tail rows this rank owns (device rows [n0, n1) of the full-length v_full), zero elsewhere
 int launch_solve_tail(const SolveArgs &a, int64_t N0, const u32 *v_full, const u32 *map, int64_t n0, int64_t n1, cudaStream_t st);
 // k_solve_small: tail, A, k -> W, found
 int launch_solve_small(const SolveArgs &a, cudaStream_t st);
-// k_solve_apply: x = v W
-int launch_solve_apply(const SolveArgs &a, cudaStream_t st);
 // prune.cu: removal of empty and singleton constraints (blk_create_pruned), DESIGN.md section 14.
 struct PruneResult {
         int64_t N = 0, Mc = 0, nnz = 0, free = 0, rounds = 0;    // kept unknowns, constraints, triplets; free unknowns; rounds

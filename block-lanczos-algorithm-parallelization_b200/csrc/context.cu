@@ -2638,63 +2638,51 @@ int blk_iterate(blk_ctx *c, int32_t max_iters, int32_t *iters_total, int32_t *st
         return 0;
 }
 
+// Host rows [0, lim) of a block along the Lanczos dimension into dst (w words per host row, wp per device row).  `own`
+// holds this rank's rows [n0, n1) (device labels); `full` (nullable) is a buffer of gather_cap(n_off) rows holding them
+// in place, else a gathered copy is made here when one is needed:
+//   relabelled rows on several GPUs: a rank's rows are scattered over the host order, so the block is gathered over
+//     NVLink (device labels) and every rank unpermutes its share [h0, h1) of HOST rows (all of them when whole)
+//   whole at world > 1 (a rank of a multi-process job must return complete blocks): gather, then every row
+//   otherwise: this rank's rows (unpermuted on the way down when one GPU holds a relabelled dimension)
+static int download_owned(blk_ctx *c, u32 *dst, int w, int wp, const u32 *own, u32 *full, int64_t lim, bool whole)
+{
+        const bool all = whole && c->world > 1;
+        const int64_t n0 = c->n0(), ln = c->n1() - n0;
+        if (!c->relabel_mg() && !all) {
+                const int64_t lo = std::min(n0, lim), hi = std::min(n0 + ln, lim);
+                return download_rows(c, dst + (size_t)lo * w, own, hi - lo, c->n_old2new, lo, w, wp);
+        }
+        u32 *copy = nullptr;
+        int rc = 0;
+        if (!full) {
+                CU(cudaMalloc(&copy, sizeof(u32) * (size_t)gather_cap(c->n_off) * wp));
+                full = copy;
+                if (cudaMemcpyAsync(full + (size_t)n0 * wp, own, sizeof(u32) * (size_t)ln * wp, cudaMemcpyDeviceToDevice,
+                                    c->stream) != cudaSuccess)
+                        rc = fail("device copy failed");
+        }
+        const int64_t r0 = all ? 0 : std::min(c->h0(), lim), r1 = all ? lim : std::min(c->h1(), lim);
+        if (!rc) rc = allgather_rows(c, full, c->n_off, wp);
+        if (!rc) rc = download_rows(c, dst + (size_t)r0 * w, full, r1 - r0, c->n_old2new, r0, w, wp);
+        cudaFree(copy);
+        return rc;
+}
+
 // What one rank contributes to blk_get_state: rows of v / Av / p straight into the caller's blocks (host layout,
 // n per row, written at their global row position) and rows of the device's tmp into `ht` (Mc x n).
 // whole = false: only this rank's rows (the blocks of a job are then assembled from the ranks' slices: group
-// contexts, blk_get_state_local); whole = true: every row -- at world > 1 the missing rows are fetched from the
-// peers over NVLink first, because a rank of a multi-process job must return complete blocks.
+// contexts, blk_get_state_local); whole = true: every row (download_owned).
 static int download_state(blk_ctx *c, u32 *v, u32 *Av, u32 *p, u32 *ht, bool whole)
 {
         CU(cudaSetDevice(c->device));
         const int n = c->geo.n, np = c->geo.np;
         if (c->grid_on && grid_export(c)) return 1;
         const bool all = whole && c->world > 1;
-        const int64_t n0 = c->n0(), ln = c->n1() - c->n0(), m0 = c->m0(), lm = c->m1() - c->m0();
-        if (c->relabel_mg()) {
-                // device labels are scattered over the host order: gather the block over NVLink (device labels), then
-                // every rank unpermutes and downloads its share of HOST rows (all of them if it must return whole blocks)
-                const int64_t r0 = all ? 0 : c->h0(), cnt = all ? c->N : c->h1() - c->h0();
-                for (int which = 0; which < 3; which++) {
-                        u32 *dst = which == 0 ? v : (which == 1 ? Av : p);
-                        if (!dst) continue;
-                        u32 *full = c->v;
-                        if (which) {
-                                CU(cudaMalloc(&full, sizeof(u32) * (size_t)gather_cap(c->n_off) * np));
-                                if (cudaMemcpyAsync(full + (size_t)n0 * np, which == 1 ? c->Av : c->p, sizeof(u32) * (size_t)ln * np,
-                                                    cudaMemcpyDeviceToDevice, c->stream) != cudaSuccess) {
-                                        cudaFree(full);
-                                        return fail("blk_get_state: device copy failed");
-                                }
-                        }
-                        int rc = allgather_rows(c, full, c->n_off);
-                        if (!rc) rc = download_rows(c, dst + (size_t)r0 * n, full, cnt, c->n_old2new, r0);
-                        if (which) cudaFree(full);
-                        if (rc) return 1;
-                }
-                v = Av = p = nullptr;                  // done
-        }
-        if (v) {
-                if (all) {
-                        if (allgather_rows(c, c->v, c->n_off)) return 1;
-                        if (download_rows(c, v, c->v, c->N)) return 1;
-                } else if (download_rows(c, v + (size_t)n0 * n, c->n_old2new ? c->v : c->v + (size_t)n0 * np, ln, c->n_old2new, n0)) return 1;
-        }
-        for (int which = 0; which < 2; which++) {
-                u32 *dst = which ? p : Av;
-                if (!dst) continue;
-                const u32 *src = which ? c->p : c->Av;                 // local rows
-                if (all) {
-                        u32 *full = nullptr;
-                        CU(cudaMalloc(&full, sizeof(u32) * (size_t)gather_cap(c->n_off) * np));
-                        int rc = 0;
-                        if (cudaMemcpyAsync(full + (size_t)n0 * np, src, sizeof(u32) * (size_t)ln * np, cudaMemcpyDeviceToDevice, c->stream) != cudaSuccess)
-                                rc = fail("blk_get_state: device copy failed");
-                        if (!rc) rc = allgather_rows(c, full, c->n_off);
-                        if (!rc) rc = download_rows(c, dst, full, c->N);
-                        cudaFree(full);
-                        if (rc) return 1;
-                } else if (download_rows(c, dst + (size_t)n0 * n, src, ln, c->n_old2new, n0)) return 1;
-        }
+        const int64_t n0 = c->n0(), m0 = c->m0(), lm = c->m1() - c->m0();
+        if (v && download_owned(c, v, n, np, c->v + (size_t)n0 * np, c->v, c->N, whole)) return 1;
+        if (Av && download_owned(c, Av, n, np, c->Av, nullptr, c->N, whole)) return 1;
+        if (p && download_owned(c, p, n, np, c->p, nullptr, c->N, whole)) return 1;
         if (ht) {
                 if (c->mg_recur && !c->ran_since_set) {
                         // nothing has run since blk_set_state: the reference's tmp is still all zero there (the
@@ -2772,6 +2760,23 @@ int blk_get_state_local(blk_ctx *c, uint32_t *v, uint32_t *Av, uint32_t *p)
         return download_state(c, v, Av, p, nullptr, false);
 }
 
+// This rank's rows [m0, m1) of T = S1 v of the current v: tmp already holds them when the loop stopped on "no pivot"
+// (or, in the multi-GPU recurrence, whenever the loop has run); otherwise S1 v goes into *scratch, allocated here and
+// freed by the caller.  v, tmp, Av and p are left as they are.
+static int rows_of_T(blk_ctx *c, const u32 **t, u32 **scratch)
+{
+        const int np = c->geo.np;
+        const int64_t lm = c->m1() - c->m0();
+        *t = c->tmp + (size_t)c->m0() * np;
+        *scratch = nullptr;
+        if (c->tmp_is_spmv || (c->mg_recur && c->ran_since_set)) return 0;
+        if (c->world > 1 && allgather_rows(c, c->v, c->n_off)) return 1;
+        CU(cudaMalloc(scratch, sizeof(u32) * (size_t)std::max<int64_t>(lm, 1) * np));
+        c->launches += launch_spmv(c->S1, c->geo, c->m, c->v, *scratch, nullptr, c->stream);
+        *t = *scratch;
+        return 0;
+}
+
 int blk_final_check(blk_ctx *c, int32_t *v_nonzero, int32_t *vtm_zero)
 {
         if (!c || !v_nonzero || !vtm_zero) return fail("blk_final_check: null argument");
@@ -2788,19 +2793,11 @@ int blk_final_check(blk_ctx *c, int32_t *v_nonzero, int32_t *vtm_zero)
         // v: every rank scans its own rows (padding columns are zero)
         if (scan_rows(c, c->v + (size_t)c->n0() * np, c->n1() - c->n0(), &nz, &big)) return 1;
         *v_nonzero = nz;
-        // tmp = S1 v of the current v: already there when the loop stopped on "no pivot" (or, in the
-        // multi-GPU recurrence, whenever the loop has run); otherwise compute it into a scratch block
-        const int64_t lm = c->m1() - c->m0();
-        bool have = c->tmp_is_spmv || (c->mg_recur && c->ran_since_set);
-        const u32 *src = c->tmp + (size_t)c->m0() * np;
+        // T = S1 v: every rank scans its own rows
+        const u32 *t = nullptr;
         u32 *scratch = nullptr;
-        if (!have) {
-                if (c->world > 1 && allgather_rows(c, c->v, c->n_off)) return 1;
-                CU(cudaMalloc(&scratch, sizeof(u32) * (size_t)(lm > 0 ? lm : 1) * np));
-                c->launches += launch_spmv(c->S1, c->geo, c->m, c->v, scratch, nullptr, c->stream);
-                src = scratch;
-        }
-        int rc = scan_rows(c, src, lm, &nz, &big);
+        if (rows_of_T(c, &t, &scratch)) return 1;
+        int rc = scan_rows(c, t, c->m1() - c->m0(), &nz, &big);
         cudaFree(scratch);
         if (rc) return 1;
         *vtm_zero = !nz;
@@ -2836,23 +2833,20 @@ int blk_check_kernel_block(blk_ctx *c, const uint32_t *x, int32_t *ok)
         return 0;
 }
 
-// One rank of blk_kernel_basis: its rows of v and T reduced to two records, the records of all ranks gathered
-// (one NCCL all-gather), the n x n stage redundantly on every rank, and X = v A_S for the rows this rank owns.
-// whole: write every row of x (a rank of a multi-process job), else only this rank's rows (group members).
-static int kernel_basis_rank(blk_ctx *c, uint32_t *x, int32_t *k, bool whole)
+// One rank of blk_kernel_basis (found == nullptr) or blk_solve: its rows of v and T reduced to two records, the records
+// of all ranks gathered (one NCCL all-gather) and the n x n stage run redundantly on every rank, giving A_S and k.  The
+// kernel basis is X = v A_S.  A solve takes the r tail rows of v from their owners (one NCCL all-reduce: every entry
+// has one owner, the others add zero), runs the r x k stage redundantly on every rank for W = A_S C and found, and
+// forms x = v W; rows from N0 = N - r on (the right-hand-side coordinates) are not part of x.  Every rank forms the
+// rows it owns.  whole: write every row of the output (a rank of a multi-process job), else only this rank's rows
+// (group members).
+static int extract_rank(blk_ctx *c, uint32_t *x, int32_t *k, int32_t *found, bool whole)
 {
         CU(cudaSetDevice(c->device));
         const int n = c->geo.n, np = c->geo.np;
+        const int r = found ? c->nrhs : 0, w = found ? r : n, wp = found ? pad_width(r) : np;
         if (c->grid_on && grid_export(c)) return 1;
         const int64_t n0 = c->n0(), ln = c->n1() - n0, lm = c->m1() - c->m0();
-        // T = S1 v of the current v, exactly as blk_final_check obtains it (v, tmp, Av and p are left as they are)
-        bool have = c->tmp_is_spmv || (c->mg_recur && c->ran_since_set);
-        const size_t rec_words = (size_t)(n + 1) * np;
-        KbArgs a;
-        a.n = n; a.world = c->world; a.m = c->m;
-        a.v = c->v + (size_t)n0 * np; a.vrows = ln;
-        a.t = c->tmp + (size_t)c->m0() * np; a.trows = lm;
-        a.ctas = kb_ctas(std::max(ln, lm));
         struct Bufs {
                 std::vector<void *> p;
                 ~Bufs() { for (void *q : p) cudaFree(q); }
@@ -2862,43 +2856,48 @@ static int kernel_basis_rank(blk_ctx *c, uint32_t *x, int32_t *k, bool whole)
                 if (e == cudaSuccess) bufs.p.push_back(*dst);
                 return e;
         };
+        KbArgs a;
+        a.n = n; a.world = c->world; a.m = c->m;
+        a.v = c->v + (size_t)n0 * np; a.vrows = ln;
+        a.trows = lm;
+        a.ctas = kb_ctas(std::max(ln, lm));
         u32 *scratch = nullptr, *xf = nullptr;
-        if (!have) {
-                if (c->world > 1 && allgather_rows(c, c->v, c->n_off)) return 1;
-                CU(grab((void **)&scratch, sizeof(u32) * (size_t)lm * np));
-                c->launches += launch_spmv(c->S1, c->geo, c->m, c->v, scratch, nullptr, c->stream);
-                a.t = scratch;
-        }
+        const int trc = rows_of_T(c, &a.t, &scratch);
+        if (scratch) bufs.p.push_back(scratch);
+        if (trc) return 1;
+        const size_t rec_words = (size_t)(n + 1) * np;
         CU(grab((void **)&a.part, sizeof(u32) * (size_t)2 * a.ctas * n * np));
         CU(grab((void **)&a.prank, sizeof(int) * (size_t)2 * a.ctas));
         CU(grab((void **)&a.counter, sizeof(unsigned)));
         CU(grab((void **)&a.rec_all, sizeof(u32) * (size_t)c->world * 2 * rec_words));
         CU(grab((void **)&a.A, sizeof(u32) * (size_t)np * np));
         CU(grab((void **)&a.k, sizeof(int)));
-        CU(grab((void **)&xf, sizeof(u32) * (size_t)gather_cap(c->n_off) * np));
+        CU(grab((void **)&xf, sizeof(u32) * (size_t)gather_cap(c->n_off) * wp));
         a.rec_own = a.rec_all + (size_t)c->rank * 2 * rec_words;
-        a.x = xf + (size_t)n0 * np;
         CU(cudaMemsetAsync(a.counter, 0, sizeof(unsigned), c->stream));
         c->launches += launch_kb_reduce(np, a, c->stream);
         if (c->world > 1)
                 NC(g_nccl.AllGather(a.rec_own, a.rec_all, 2 * rec_words, ncclUint32, c->comm, c->stream));
         c->launches += launch_kb_small(np, a, c->stream);
-        c->launches += launch_kb_apply(np, a, c->stream);
-        int hk = 0;
-        CU(cudaMemcpyAsync(&hk, a.k, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+        SolveArgs s;
+        s.W = a.A;
+        if (found) {
+                s.np = np; s.r = r; s.rp = wp; s.m = c->m; s.A = a.A; s.k = a.k;
+                CU(grab((void **)&s.tail, sizeof(u32) * (size_t)r * np));
+                CU(grab((void **)&s.W, sizeof(u32) * (size_t)np * wp));
+                CU(grab((void **)&s.found, sizeof(int) * (size_t)r));
+                c->launches += launch_solve_tail(s, c->N - r, c->v, c->n_old2new, n0, n0 + ln, c->stream);
+                if (c->world > 1)
+                        NC(g_nccl.AllReduce(s.tail, s.tail, (size_t)r * np, ncclUint32, ncclSum, c->comm, c->stream));
+                c->launches += launch_solve_small(s, c->stream);
+        }
+        c->launches += launch_block_apply(np, wp, ln, a.v, s.W, xf + (size_t)n0 * wp, c->m, c->stream);
+        std::vector<int> h((size_t)(found ? r : 1), 0);
+        CU(cudaMemcpyAsync(h.data(), found ? s.found : a.k, sizeof(int) * h.size(), cudaMemcpyDeviceToHost, c->stream));
         CU(cudaStreamSynchronize(c->stream));
         CU(cudaGetLastError());
-        // down to the host like v in download_state
-        const bool all = whole && c->world > 1;
-        if (c->relabel_mg()) {
-                const int64_t r0 = all ? 0 : c->h0(), cnt = all ? c->N : c->h1() - c->h0();
-                if (allgather_rows(c, xf, c->n_off)) return 1;
-                if (download_rows(c, x + (size_t)r0 * n, xf, cnt, c->n_old2new, r0)) return 1;
-        } else if (all) {
-                if (allgather_rows(c, xf, c->n_off)) return 1;
-                if (download_rows(c, x, xf, c->N)) return 1;
-        } else if (download_rows(c, x + (size_t)n0 * n, c->n_old2new ? xf : xf + (size_t)n0 * np, ln, c->n_old2new, n0)) return 1;
-        *k = hk;
+        if (download_owned(c, x, w, wp, xf + (size_t)n0 * wp, xf, c->N - r, whole)) return 1;
+        std::copy(h.begin(), h.end(), found ? found : k);
         return 0;
 }
 
@@ -2908,91 +2907,11 @@ int blk_kernel_basis(blk_ctx *c, uint32_t *x, int32_t *k)
         if (c->is_group()) {
                 // every GPU writes its own rows into the one host block
                 std::vector<int32_t> kk(c->members.size(), 0);
-                if (group_run(c, [&](blk_ctx *mem, int r) { return kernel_basis_rank(mem, x, &kk[(size_t)r], false); })) return 1;
+                if (group_run(c, [&](blk_ctx *mem, int r) { return extract_rank(mem, x, &kk[(size_t)r], nullptr, false); })) return 1;
                 *k = kk[0];
                 return 0;
         }
-        return kernel_basis_rank(c, x, k, true);
-}
-
-// One rank of blk_solve: A_S and k exactly as kernel_basis_rank obtains them, the r tail rows of v from their owners
-// (one NCCL all-reduce: every entry has one owner, the others add zero), the r x k stage redundantly on every rank,
-// and x = v W for the rows this rank owns.  whole: as in kernel_basis_rank.  Rows from N0 = N - r on (the
-// right-hand-side coordinates) are not part of x.
-static int solve_rank(blk_ctx *c, uint32_t *x, int32_t *found, bool whole)
-{
-        CU(cudaSetDevice(c->device));
-        const int n = c->geo.n, np = c->geo.np, r = c->nrhs, rp = pad_width(r);
-        if (c->grid_on && grid_export(c)) return 1;
-        const int64_t n0 = c->n0(), ln = c->n1() - n0, lm = c->m1() - c->m0(), N0 = c->N - r;
-        bool have = c->tmp_is_spmv || (c->mg_recur && c->ran_since_set);
-        const size_t rec_words = (size_t)(n + 1) * np;
-        KbArgs a;
-        a.n = n; a.world = c->world; a.m = c->m;
-        a.v = c->v + (size_t)n0 * np; a.vrows = ln;
-        a.t = c->tmp + (size_t)c->m0() * np; a.trows = lm;
-        a.ctas = kb_ctas(std::max(ln, lm));
-        struct Bufs {
-                std::vector<void *> p;
-                ~Bufs() { for (void *q : p) cudaFree(q); }
-        } bufs;
-        auto grab = [&](void **dst, size_t bytes) {
-                cudaError_t e = cudaMalloc(dst, bytes ? bytes : 4);
-                if (e == cudaSuccess) bufs.p.push_back(*dst);
-                return e;
-        };
-        u32 *scratch = nullptr, *xf = nullptr;
-        if (!have) {
-                if (c->world > 1 && allgather_rows(c, c->v, c->n_off)) return 1;
-                CU(grab((void **)&scratch, sizeof(u32) * (size_t)lm * np));
-                c->launches += launch_spmv(c->S1, c->geo, c->m, c->v, scratch, nullptr, c->stream);
-                a.t = scratch;
-        }
-        CU(grab((void **)&a.part, sizeof(u32) * (size_t)2 * a.ctas * n * np));
-        CU(grab((void **)&a.prank, sizeof(int) * (size_t)2 * a.ctas));
-        CU(grab((void **)&a.counter, sizeof(unsigned)));
-        CU(grab((void **)&a.rec_all, sizeof(u32) * (size_t)c->world * 2 * rec_words));
-        CU(grab((void **)&a.A, sizeof(u32) * (size_t)np * np));
-        CU(grab((void **)&a.k, sizeof(int)));
-        a.rec_own = a.rec_all + (size_t)c->rank * 2 * rec_words;
-        SolveArgs s;
-        s.np = np; s.r = r; s.rp = rp; s.m = c->m; s.A = a.A; s.k = a.k;
-        s.v = a.v; s.vrows = ln;
-        CU(grab((void **)&s.tail, sizeof(u32) * (size_t)r * np));
-        CU(grab((void **)&s.W, sizeof(u32) * (size_t)np * rp));
-        CU(grab((void **)&s.found, sizeof(int) * (size_t)r));
-        CU(grab((void **)&xf, sizeof(u32) * (size_t)gather_cap(c->n_off) * rp));
-        s.x = xf + (size_t)n0 * rp;
-        CU(cudaMemsetAsync(a.counter, 0, sizeof(unsigned), c->stream));
-        c->launches += launch_kb_reduce(np, a, c->stream);
-        if (c->world > 1)
-                NC(g_nccl.AllGather(a.rec_own, a.rec_all, 2 * rec_words, ncclUint32, c->comm, c->stream));
-        c->launches += launch_kb_small(np, a, c->stream);
-        c->launches += launch_solve_tail(s, N0, c->v, c->n_old2new, n0, n0 + ln, c->stream);
-        if (c->world > 1)
-                NC(g_nccl.AllReduce(s.tail, s.tail, (size_t)r * np, ncclUint32, ncclSum, c->comm, c->stream));
-        c->launches += launch_solve_small(s, c->stream);
-        c->launches += launch_solve_apply(s, c->stream);
-        std::vector<int> hf((size_t)r, 0);
-        CU(cudaMemcpyAsync(hf.data(), s.found, sizeof(int) * (size_t)r, cudaMemcpyDeviceToHost, c->stream));
-        CU(cudaStreamSynchronize(c->stream));
-        CU(cudaGetLastError());
-        // down to the host like X in kernel_basis_rank, host rows [0, N0) only
-        const bool all = whole && c->world > 1;
-        if (c->relabel_mg()) {
-                const int64_t r0 = all ? 0 : std::min(c->h0(), N0), r1 = all ? N0 : std::min(c->h1(), N0);
-                if (allgather_rows(c, xf, c->n_off, rp)) return 1;
-                if (download_rows(c, x + (size_t)r0 * r, xf, r1 - r0, c->n_old2new, r0, r, rp)) return 1;
-        } else if (all) {
-                if (allgather_rows(c, xf, c->n_off, rp)) return 1;
-                if (download_rows(c, x, xf, N0, nullptr, 0, r, rp)) return 1;
-        } else {
-                const int64_t lo = std::min(n0, N0), hi = std::min(n0 + ln, N0);
-                if (download_rows(c, x + (size_t)lo * r, c->n_old2new ? xf : xf + (size_t)lo * rp, hi - lo, c->n_old2new, lo, r, rp))
-                        return 1;
-        }
-        for (int j = 0; j < r; j++) found[j] = hf[(size_t)j];
-        return 0;
+        return extract_rank(c, x, k, nullptr, true);
 }
 
 int blk_solve(blk_ctx *c, uint32_t *x, int32_t *found)
@@ -3002,11 +2921,11 @@ int blk_solve(blk_ctx *c, uint32_t *x, int32_t *found)
         if (c->is_group()) {
                 // every GPU writes its own rows into the one host block
                 std::vector<std::vector<int32_t>> ff(c->members.size(), std::vector<int32_t>((size_t)c->nrhs, 0));
-                if (group_run(c, [&](blk_ctx *mem, int r) { return solve_rank(mem, x, ff[(size_t)r].data(), false); })) return 1;
+                if (group_run(c, [&](blk_ctx *mem, int r) { return extract_rank(mem, x, nullptr, ff[(size_t)r].data(), false); })) return 1;
                 for (int j = 0; j < c->nrhs; j++) found[j] = ff[0][(size_t)j];
                 return 0;
         }
-        return solve_rank(c, x, found, true);
+        return extract_rank(c, x, nullptr, found, true);
 }
 
 int blk_get_small(blk_ctx *c, uint32_t *vtAv, uint32_t *vtAAv, uint32_t *winv, uint32_t *d, int32_t *npiv)

@@ -12,7 +12,8 @@
 //                 bases into this rank's basis of each block (a "record": rank word, then the rows)
 //   k_kb_small    one CTA: merges the records of all ranks (gathered), then steps E_T, a_f, B, S above; writes the
 //                 n_pad x n_pad matrix A_S (column s = a_f of the s-th f in S, zero columns from k on) and k
-//   k_kb_apply    X = v A_S row by row, with the row x (n x n) code of orthogonalize (dense_body.cuh: ortho_slot)
+//   k_block_apply x = v W for an n_pad x w_pad matrix W, one multiply-add per product: X = v A_S here, x = v (A_S C) for
+//                 blk_solve (solve.cu)
 //
 // Every product is accumulated lazily in u64 (mp_mac / mp_fold of modp.cuh), exact for every 2 <= p < 2^31.
 #include "blk_internal.cuh"
@@ -310,20 +311,58 @@ k_kb_small(const u32 *rec, int world, int n, u32 *A_out, int *k_out, ModP m)
         }
 }
 
-// X = v A_S with the row code of orthogonalize: its p' = v Wm + (d ? 0 : p) is v A_S for Wm = A_S and every d non-zero.
-// Its v' (v C + p D + Av, here with C = D = 0) goes to the same row of x first and is overwritten by p'.
-constexpr int KB_APPLY_TB = 128;
+// x = v W (W: NP x WP, WP <= NP): thread (row, slice) forms OC consecutive outputs of one row from the whole row of v
+// (NP words, vector loads) and W in shared memory; every product is one multiply-add into a lazy u64, folded every FOLD
+// products (0: never, NP <= 64 products fit).
+constexpr int APPLY_TB = 256;
 
-template <int NP, int JT, int FOLD>
-__global__ void __launch_bounds__(KB_APPLY_TB)
-k_kb_apply(int64_t rows, const u32 *v, u32 *x, const u32 *A, ModP m)
+template <int NP, int WP, int FOLD>
+__global__ void __launch_bounds__(APPLY_TB)
+k_block_apply(int64_t rows, const u32 *__restrict__ v, const u32 *__restrict__ W, u32 *__restrict__ x, ModP m)
 {
-        extern __shared__ u32 sm_ap[];
-        u32 *Cz = sm_ap, *Dz = Cz + NP * NP, *Wm = Dz + NP * NP, *dm = Wm + NP * NP;
-        for (int e = threadIdx.x; e < NP * NP; e += KB_APPLY_TB) { Cz[e] = 0; Dz[e] = 0; Wm[e] = A[e]; }
-        for (int e = threadIdx.x; e < NP; e += KB_APPLY_TB) dm[e] = 1;
+        constexpr int OC = WP < 8 ? WP : 8;               // outputs per thread
+        constexpr int TPR = WP / OC;                      // threads per row
+        constexpr int VL = NP < 4 ? NP : 4;               // words per load
+        __shared__ u32 Ws[NP * WP];
+        for (int e = threadIdx.x; e < NP * WP; e += APPLY_TB) Ws[e] = W[e];
         __syncthreads();
-        ortho_slot<NP, JT, FOLD, 0>((int64_t)blockIdx.x * KB_APPLY_TB + threadIdx.x, rows, v, v, v, x, x, Cz, Dz, Wm, dm, m);
+        const int64_t gid = (int64_t)blockIdx.x * APPLY_TB + threadIdx.x;
+        const int64_t row = gid / TPR;
+        if (row >= rows) return;
+        const int o0 = (int)(gid % TPR) * OC;
+        u64 acc[OC];
+#pragma unroll
+        for (int o = 0; o < OC; o++) acc[o] = 0;
+        const u32 *vr = v + row * NP;
+#pragma unroll
+        for (int j0 = 0; j0 < NP; j0 += VL) {
+                u32 a[VL];
+                ldv<VL>(a, vr + j0);
+#pragma unroll
+                for (int jj = 0; jj < VL; jj++) {
+#pragma unroll
+                        for (int o = 0; o < OC; o++) mp_mac(acc[o], a[jj], Ws[(j0 + jj) * WP + o0 + o]);
+                        if constexpr (FOLD > 0) {
+                                if ((j0 + jj + 1) % FOLD == 0) {
+#pragma unroll
+                                        for (int o = 0; o < OC; o++) mp_fold(acc[o], m);
+                                }
+                        }
+                }
+        }
+        u32 out[OC];
+#pragma unroll
+        for (int o = 0; o < OC; o++) out[o] = mp_reduce(acc[o], m);
+        u32 *xr = x + row * WP + o0;
+        if constexpr (OC >= 4) {
+#pragma unroll
+                for (int o = 0; o < OC; o += 4) {
+                        u32 w4[4] = {out[o], out[o + 1], out[o + 2], out[o + 3]};
+                        stv<4>(xr + o, w4);
+                }
+        } else {
+                stv<OC>(xr, out);
+        }
 }
 
 template <int NP>
@@ -347,23 +386,32 @@ int small_go(const KbArgs &a, cudaStream_t st)
         return 1;
 }
 
-template <int NP, int JT>
-int apply_go(const KbArgs &a, cudaStream_t st)
+template <int NP, int WP>
+int apply_wp(int64_t rows, const u32 *v, const u32 *W, u32 *x, const ModP &m, cudaStream_t st)
 {
-        if (a.vrows <= 0) return 0;
-        const size_t smem = sizeof(u32) * (3 * NP * NP + NP);
-        const int64_t threads = a.vrows * (NP / JT);
-        const unsigned blocks = (unsigned)((threads + KB_APPLY_TB - 1) / KB_APPLY_TB);
-        auto go = [&](auto kern) {
-                cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                kern<<<blocks, KB_APPLY_TB, smem, st>>>(a.vrows, a.v, a.x, a.A, a.m);
-        };
-        switch (a.m.fold_every) {
-        case 0: go(k_kb_apply<NP, JT, 0>); break;
-        case 8: go(k_kb_apply<NP, JT, 8>); break;
-        default: go(k_kb_apply<NP, JT, 2>); break;
+        constexpr int OC = WP < 8 ? WP : 8, TPR = WP / OC;
+        const unsigned blocks = (unsigned)((rows * TPR + APPLY_TB - 1) / APPLY_TB);
+        switch (m.fold_every) {
+        case 0: k_block_apply<NP, WP, 0><<<blocks, APPLY_TB, 0, st>>>(rows, v, W, x, m); break;
+        case 8: k_block_apply<NP, WP, 8><<<blocks, APPLY_TB, 0, st>>>(rows, v, W, x, m); break;
+        default: k_block_apply<NP, WP, 2><<<blocks, APPLY_TB, 0, st>>>(rows, v, W, x, m); break;
         }
         return 1;
+}
+
+template <int NP>
+int apply_np(int wp, int64_t rows, const u32 *v, const u32 *W, u32 *x, const ModP &m, cudaStream_t st)
+{
+        switch (wp) {
+        case 1: return apply_wp<NP, 1>(rows, v, W, x, m, st);
+        case 2: if constexpr (NP >= 2) return apply_wp<NP, 2>(rows, v, W, x, m, st); break;
+        case 4: if constexpr (NP >= 4) return apply_wp<NP, 4>(rows, v, W, x, m, st); break;
+        case 8: if constexpr (NP >= 8) return apply_wp<NP, 8>(rows, v, W, x, m, st); break;
+        case 16: if constexpr (NP >= 16) return apply_wp<NP, 16>(rows, v, W, x, m, st); break;
+        case 32: if constexpr (NP >= 32) return apply_wp<NP, 32>(rows, v, W, x, m, st); break;
+        case 64: if constexpr (NP >= 64) return apply_wp<NP, 64>(rows, v, W, x, m, st); break;
+        }
+        return -1;
 }
 
 }  // namespace
@@ -404,16 +452,17 @@ int launch_kb_small(int np, const KbArgs &a, cudaStream_t st)
         return -1;
 }
 
-int launch_kb_apply(int np, const KbArgs &a, cudaStream_t st)
+int launch_block_apply(int np, int wp, int64_t rows, const u32 *v, const u32 *W, u32 *x, const ModP &m, cudaStream_t st)
 {
+        if (rows <= 0) return 0;
         switch (np) {
-        case 1: return apply_go<1, 1>(a, st);
-        case 2: return apply_go<2, 2>(a, st);
-        case 4: return apply_go<4, 4>(a, st);
-        case 8: return apply_go<8, 8>(a, st);
-        case 16: return apply_go<16, 16>(a, st);
-        case 32: return apply_go<32, 16>(a, st);
-        case 64: return apply_go<64, 16>(a, st);
+        case 1: return apply_np<1>(wp, rows, v, W, x, m, st);
+        case 2: return apply_np<2>(wp, rows, v, W, x, m, st);
+        case 4: return apply_np<4>(wp, rows, v, W, x, m, st);
+        case 8: return apply_np<8>(wp, rows, v, W, x, m, st);
+        case 16: return apply_np<16>(wp, rows, v, W, x, m, st);
+        case 32: return apply_np<32>(wp, rows, v, W, x, m, st);
+        case 64: return apply_np<64>(wp, rows, v, W, x, m, st);
         }
         return -1;
 }

@@ -13,12 +13,11 @@
 //   k_solve_tail                   the r tail rows of v that this rank owns (an r x n_pad block, zero elsewhere;
 //                                  the ranks' blocks are summed by one all-reduce)
 //   k_solve_small                  one CTA: T = v_tail A_S, Gauss-Jordan of [T | I_r], C, W = A_S C, found
-//   k_solve_apply                  x = v W, r_pad output columns, one lazy u64 multiply-add per product
 //
-// A_S and k come from k_kb_reduce / k_kb_small of kernel_basis.cu, unchanged.
+// A_S and k come from k_kb_reduce / k_kb_small of kernel_basis.cu, unchanged; x = v W is its k_block_apply with r_pad
+// output columns.
 #include <cub/cub.cuh>
 #include "blk_internal.cuh"
-#include "dense_body.cuh"
 
 namespace {
 
@@ -166,90 +165,6 @@ k_solve_small(const u32 *__restrict__ A, const int *__restrict__ k_in, const u32
         }
 }
 
-// x = v W: thread (row, slice) forms OC consecutive outputs of one row from the whole row of v (NP words, vector
-// loads) and W in shared memory; every product is one multiply-add into a lazy u64, folded every FOLD products
-// (0: never, NP <= 64 products fit).
-constexpr int APPLY_TB = 256;
-
-template <int NP, int RP, int FOLD>
-__global__ void __launch_bounds__(APPLY_TB)
-k_solve_apply(int64_t rows, const u32 *__restrict__ v, const u32 *__restrict__ W, u32 *__restrict__ x, ModP m)
-{
-        constexpr int OC = RP < 8 ? RP : 8;               // outputs per thread
-        constexpr int TPR = RP / OC;                      // threads per row
-        constexpr int VL = NP < 4 ? NP : 4;               // words per load
-        __shared__ u32 Ws[NP * RP];
-        for (int e = threadIdx.x; e < NP * RP; e += APPLY_TB) Ws[e] = W[e];
-        __syncthreads();
-        const int64_t gid = (int64_t)blockIdx.x * APPLY_TB + threadIdx.x;
-        const int64_t row = gid / TPR;
-        if (row >= rows) return;
-        const int o0 = (int)(gid % TPR) * OC;
-        u64 acc[OC];
-#pragma unroll
-        for (int o = 0; o < OC; o++) acc[o] = 0;
-        const u32 *vr = v + row * NP;
-#pragma unroll
-        for (int j0 = 0; j0 < NP; j0 += VL) {
-                u32 a[VL];
-                ldv<VL>(a, vr + j0);
-#pragma unroll
-                for (int jj = 0; jj < VL; jj++) {
-#pragma unroll
-                        for (int o = 0; o < OC; o++) mp_mac(acc[o], a[jj], Ws[(j0 + jj) * RP + o0 + o]);
-                        if constexpr (FOLD > 0) {
-                                if ((j0 + jj + 1) % FOLD == 0) {
-#pragma unroll
-                                        for (int o = 0; o < OC; o++) mp_fold(acc[o], m);
-                                }
-                        }
-                }
-        }
-        u32 out[OC];
-#pragma unroll
-        for (int o = 0; o < OC; o++) out[o] = mp_reduce(acc[o], m);
-        u32 *xr = x + row * RP + o0;
-        if constexpr (OC >= 4) {
-#pragma unroll
-                for (int o = 0; o < OC; o += 4) {
-                        u32 w4[4] = {out[o], out[o + 1], out[o + 2], out[o + 3]};
-                        stv<4>(xr + o, w4);
-                }
-        } else {
-                stv<OC>(xr, out);
-        }
-}
-
-template <int NP, int RP>
-int apply_rp(const SolveArgs &a, cudaStream_t st)
-{
-        constexpr int OC = RP < 8 ? RP : 8, TPR = RP / OC;
-        const int64_t threads = a.vrows * TPR;
-        const unsigned blocks = (unsigned)((threads + APPLY_TB - 1) / APPLY_TB);
-        switch (a.m.fold_every) {
-        case 0: k_solve_apply<NP, RP, 0><<<blocks, APPLY_TB, 0, st>>>(a.vrows, a.v, a.W, a.x, a.m); break;
-        case 8: k_solve_apply<NP, RP, 8><<<blocks, APPLY_TB, 0, st>>>(a.vrows, a.v, a.W, a.x, a.m); break;
-        default: k_solve_apply<NP, RP, 2><<<blocks, APPLY_TB, 0, st>>>(a.vrows, a.v, a.W, a.x, a.m); break;
-        }
-        return 1;
-}
-
-template <int NP>
-int apply_np(const SolveArgs &a, cudaStream_t st)
-{
-        if (a.vrows <= 0) return 0;
-        switch (a.rp) {
-        case 1: return apply_rp<NP, 1>(a, st);
-        case 2: if constexpr (NP >= 2) return apply_rp<NP, 2>(a, st); break;
-        case 4: if constexpr (NP >= 4) return apply_rp<NP, 4>(a, st); break;
-        case 8: if constexpr (NP >= 8) return apply_rp<NP, 8>(a, st); break;
-        case 16: if constexpr (NP >= 16) return apply_rp<NP, 16>(a, st); break;
-        case 32: if constexpr (NP >= 32) return apply_rp<NP, 32>(a, st); break;
-        case 64: if constexpr (NP >= 64) return apply_rp<NP, 64>(a, st); break;
-        }
-        return -1;
-}
-
 template <int NP>
 int small_np(const SolveArgs &a, cudaStream_t st)
 {
@@ -321,20 +236,6 @@ int launch_solve_small(const SolveArgs &a, cudaStream_t st)
         case 16: return small_np<16>(a, st);
         case 32: return small_np<32>(a, st);
         case 64: return small_np<64>(a, st);
-        }
-        return -1;
-}
-
-int launch_solve_apply(const SolveArgs &a, cudaStream_t st)
-{
-        switch (a.np) {
-        case 1: return apply_np<1>(a, st);
-        case 2: return apply_np<2>(a, st);
-        case 4: return apply_np<4>(a, st);
-        case 8: return apply_np<8>(a, st);
-        case 16: return apply_np<16>(a, st);
-        case 32: return apply_np<32>(a, st);
-        case 64: return apply_np<64>(a, st);
         }
         return -1;
 }

@@ -85,10 +85,10 @@ def main():
             if ev.device_type is not None and "CUDA" in str(ev.device_type) and ev.self_device_time_total > 0:
                 nm = ev.key
                 tag = ("k_kb_reduce" if "k_kb_reduce" in nm else "k_kb_small" if "k_kb_small" in nm else
-                       "k_kb_apply" if "k_kb_apply" in nm else "spmv (T = M^T v)" if "spmv" in nm else
+                       "k_block_apply" if "k_block_apply" in nm else "spmv (T = M^T v)" if "spmv" in nm else
                        "unpad (host layout)" if "unpad" in nm else "other")
                 kern[tag] = kern.get(tag, 0.0) + ev.self_device_time_total / 1000.0
-        kb_ms = sum(kern.get(t, 0.0) for t in ("k_kb_reduce", "k_kb_small", "k_kb_apply"))
+        kb_ms = sum(kern.get(t, 0.0) for t in ("k_kb_reduce", "k_kb_small", "k_block_apply"))
         rd, wr = (N + Mc) * npad * 4, N * n * 4
         best = min(times)
         res["states"][name] = dict(

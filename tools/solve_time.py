@@ -8,7 +8,7 @@ bench.py config-4 matrix (50M x 50M power law) with dense random right-hand side
 For each: ms per iteration of the loop on the augmented matrix against the plain matrix at the same n and p (CUDA
 events around blk_iterate, after a warm-up), the whole blk_solve call (CUDA events, after a warm-up call; it includes
 T = M^T v and the copy of x to the host), and the device time of its kernels from torch.profiler in a separate call.
-k_solve_apply is set against the copy-rate floor: the bytes it has to move (N n_pad 4 read, N r_pad 4 written) at the
+k_block_apply is set against the copy-rate floor: the bytes it has to move (N n_pad 4 read, N r_pad 4 written) at the
 device-to-device copy rate measured in the same run.  The card's name and power limit are read in the same run.
 
     python tools/solve_time.py --out /tmp/solve_time.json [--iters 8] [--reps 3]
@@ -31,7 +31,7 @@ STATES = {
     "cfg4_r8": dict(n=16, p=2147483647, r=8),
     "p2n64_r8": dict(n=64, p=2, r=8),
 }
-TAGS = ("k_kb_reduce", "k_kb_small", "k_solve_tail", "k_solve_small", "k_solve_apply")
+TAGS = ("k_kb_reduce", "k_kb_small", "k_solve_tail", "k_solve_small", "k_block_apply")
 
 
 def card():
@@ -158,7 +158,7 @@ def main():
             iteration_ratio=ms_it / plain["ms_per_iteration"],
             call_ms=times, call_ms_best=min(times), device_kernels_ms=kern, solve_kernels_ms=solve_ms,
             apply_bytes=apply_bytes, apply_copy_floor_ms=floor_ms,
-            apply_share_of_copy_floor=floor_ms / kern["k_solve_apply"] if kern.get("k_solve_apply") else None)
+            apply_share_of_copy_floor=floor_ms / kern["k_block_apply"] if kern.get("k_block_apply") else None)
         print(name, json.dumps(res["states"][name]), flush=True)
         ctx.close()
         del x
